@@ -14,7 +14,13 @@ tangential, robust (Cauchy 0.5), poses + points refined, micro-lens-centre adjus
 is the N=1 workload too; with N GPUs the same scene is sharded by point/frame range (strong scaling).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg4|cfg3|cfg2|cfg1]
+                  [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...      (one rank per GPU, NCCL)
+
+--dump-outputs DIR writes what the last timed solve returned to its caller as float64 .npy files: camera.npy (17),
+views.npy (F x 6), points.npy (P x 3; with N ranks points_rank<r>.npy, the point range of rank r) and iteration_cost.npy
+(the cost of every LM row). The scene comes from a fixed seed, so two builds run with the same arguments can be compared
+output for output. cfg4, the largest workload, writes 24 MB.
 """
 from __future__ import annotations
 
@@ -174,6 +180,19 @@ def host_threads() -> int:
     return max(ob.max_threads(), ncores)
 
 
+def dump_outputs(out_dir: str, **arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy in float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+
+def solve_outputs(camera, views, points, summary, lo=0, hi=None) -> dict:
+    """What a solve returns to its caller, in the shapes --dump-outputs writes; points lo:hi only (a rank's range)."""
+    return {"camera": camera, "views": np.reshape(views, (-1, 6)), "points": np.reshape(points, (-1, 3))[lo:hi],
+            "iteration_cost": [r["cost"] for r in summary["iterations"]]}
+
+
 def run_cpu_baseline(workload: str, lm_iterations: int | None, scene=None, repeats: int = 1, warmup: int = 0):
     """Times the oracle on the benchmarked scene itself. cfg1-cfg3: the complete solve. cfg4 (1.12e8 observations, about
     35 s per Jacobian pass on 16 cores): a solve TRUNCATED after `lm_iterations` LM iterations — every Ceres iteration
@@ -193,8 +212,8 @@ def run_cpu_baseline(workload: str, lm_iterations: int | None, scene=None, repea
     dt, evals, rows = 0.0, 0, 0
     for k in range(warmup + repeats):
         t0 = time.perf_counter()
-        _, _, _, s = ob.solve(pa, scene.camera_init, scene.views_init, scene.points_init, options=opts, threads=threads,
-                              streaming=streaming)
+        cam, vw, pt, s = ob.solve(pa, scene.camera_init, scene.views_init, scene.points_init, options=opts, threads=threads,
+                                  streaming=streaming)
         if k >= warmup:
             dt += time.perf_counter() - t0
             evals += s["num_jacobian_evals"]
@@ -208,7 +227,7 @@ def run_cpu_baseline(workload: str, lm_iterations: int | None, scene=None, repea
             "lm_iters_per_s": max(0, rows - repeats) / dt, "seconds": dt, "n_obs": n, "lm_rows": rows, "repeats": repeats,
             "warmup": warmup,
             "jacobian_evals": evals, "same_scene": True, "oracle_mode": "streaming" if streaming else "stored",
-            "final_cost": s["final_cost"]}
+            "final_cost": s["final_cost"], "outputs": solve_outputs(cam, vw, pt, s)}
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -223,7 +242,11 @@ def main():
     ap.add_argument("--cpu-iterations", type=int, default=3,
                     help="cfg4 only: LM iterations of the CPU solve that --impl reference times (the scene is the full one)")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed solve returned as DIR/<name>.npy (float64; see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
 
     # The contract is ONE JSON line on stdout. Libraries write banners there (NCCL prints its version at communicator
     # creation): everything but the final line goes to stderr.
@@ -245,20 +268,20 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return 0
-        small = args.workload in ("cfg1", "cfg2")
+        # cfg4: a CPU step takes minutes (1.12e8 observations); choose a small --steps there
         iters = None if args.workload != "cfg4" else args.cpu_iterations
-        reps, wu = (max(1, min(args.steps, 3)), min(1, args.warmup)) if small else (1, 0)
-        cb = run_cpu_baseline(args.workload, iters, repeats=reps, warmup=wu)
+        cb = run_cpu_baseline(args.workload, iters, repeats=args.steps, warmup=args.warmup)
         line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
-                "steps": reps, "warmup": wu, "requested_steps": args.steps, "requested_warmup": args.warmup,
+                "steps": args.steps, "warmup": args.warmup,
                 "steps_note": "a step is one LM solve of the FULL benchmarked scene on the host cores (cfg4: truncated after "
-                              "--cpu-iterations LM iterations; the rate extrapolates); K repetitions of a 1.12e8-observation "
-                              "CPU solve would take hours, so fewer steps than requested are timed",
-                "ms_per_step": 1e3 * cb["seconds"] / reps, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
+                              "--cpu-iterations LM iterations; the rate extrapolates)",
+                "ms_per_step": 1e3 * cb["seconds"] / args.steps, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
                 "dtype": "f64", "data": "synthetic", "config": config, "lm_iters_per_s": cb["lm_iters_per_s"],
                 "cpu_baseline": {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample", "same_scene", "oracle_mode")},
                 "e2e": {"value": cb["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
                 "final_cost": cb["final_cost"], "gpu_launches": 0}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, **cb["outputs"])
         emit(line)
         return 0
 
@@ -324,6 +347,8 @@ def main():
     barrier()
     wall = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
+    # read back before time_eval below evaluates on the same session
+    outputs = solve_outputs(*ds.get_parameters(), s, lo, hi) if args.dump_outputs else None
     if dist is not None:
         t = torch.tensor([gpu_ms, wall], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -383,7 +408,7 @@ def main():
             pin_par = [torch.empty(n_, dtype=torch.float64).pin_memory()
                        for n_ in (17, sc.views_init.size, sc.points_init.size)]
             par = [t_.numpy() for t_ in pin_par]
-            for k in range(1 + min(2, args.steps)):
+            for k in range(1 + args.steps):
                 for dst, src in zip(par, (sc.camera_init, sc.views_init, sc.points_init)):
                     dst[:] = np.asarray(src, np.float64).ravel()
                 barrier()
@@ -396,7 +421,7 @@ def main():
                     ev2 += s2["num_jacobian_evals"]
                     h2d.append(s2.get("h2d_gbs"))
         else:
-            for k in range(1 + min(2, args.steps)):
+            for k in range(1 + args.steps):
                 barrier()
                 t1 = time.perf_counter()
                 d2 = api.DeviceSolver(ppa, o2, communicator=comm)
@@ -421,6 +446,11 @@ def main():
 
     if comm is not None:
         comm.close()
+    if outputs is not None:
+        if world > 1:  # every rank writes the points of its own range; camera, views and rows are the same on all ranks
+            mine = {f"points_rank{rank}": outputs.pop("points")}
+            outputs = dict(outputs, **mine) if rank == 0 else mine
+        dump_outputs(args.dump_outputs, **outputs)
     if rank != 0:
         if dist is not None:
             dist.barrier()

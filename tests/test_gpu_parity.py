@@ -447,7 +447,7 @@ def test_recalib_shards_emulated(gpu):
 def test_in_process_multi_gpu_solve(gpu):
     """lfba_solve(num_gpus = 2): one host thread per GPU, NCCL all-reduce of the partial systems."""
     if api.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     sc = capi.make_scene(None, n_points=1500, n_frames=64, window=4, seed=77, order=1)
     init = (sc.camera_init, sc.views_init, sc.points_init)
     one = api.solve(sc.problem, *init)

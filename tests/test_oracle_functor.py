@@ -14,6 +14,7 @@ from lifcal_b200 import capi
 from oracle import binding as ob
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "functor_kat.npz")
+NO_REF = "oracle/_ref not built: needs the upstream LiFCal sources (make -C oracle ref REF=<LiFCal checkout>)"
 ARITY_BITS = [capi.CFG_REFINE_POSES | capi.CFG_REFINE_POINTS, capi.CFG_REFINE_POSES, 0]
 
 
@@ -47,7 +48,7 @@ def test_oracle_matches_reference_golden(built):
     assert checked == 12 * 3 * 2
 
 
-@pytest.mark.skipif(ob.ref_lib() is None, reason="oracle/_ref not built (needs /root/reference)")
+@pytest.mark.skipif(ob.ref_lib() is None, reason=NO_REF)
 def test_oracle_matches_reference_live(built):
     rng = np.random.default_rng(7)
     worst = 0.0
@@ -119,7 +120,7 @@ def test_oracle_jacobian_vs_finite_differences(built):
         assert np.max(np.abs(fd - an)) <= 2e-5 * (1 + np.max(np.abs(an))), j
 
 
-@pytest.mark.skipif(ob.ref_lib() is None, reason="oracle/_ref not built (needs /root/reference)")
+@pytest.mark.skipif(ob.ref_lib() is None, reason=NO_REF)
 def test_pose_matrix_matches_reference(built):
     R = ob.ref_lib()
     rng = np.random.default_rng(5)

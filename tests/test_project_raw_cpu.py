@@ -13,7 +13,7 @@ from oracle import binding as ob
 def test_epipolar_primitives_equal_the_reference_class_bit_for_bit(built):
     R = ob.ref_lib()
     if R is None or not hasattr(R, "ref_epi_make"):
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+        pytest.skip("oracle/_ref not built: needs the upstream LiFCal sources (make -C oracle ref REF=<LiFCal checkout>)")
     L = ob.lib()
     rng = np.random.default_rng(5)
     a, b, o, r = (np.zeros(3) for _ in range(4))
