@@ -307,6 +307,38 @@ int lfba_solver_time_eval(lfba_solver* s, int reps, int materialize, double* mea
  * Single-shard sessions only. */
 int lfba_solver_track_blocks(lfba_solver* s, int64_t* n_tracks, int32_t* rec_stride, double* rec, double* camsum64,
                              int32_t* trk_point, int32_t* trk_frame);
+/* ---- parameter covariance (ceres::Covariance of the camera and pose blocks) ----
+ * Sigma = (J^T W J)^-1 of the free parameters at the given / accepted parameters, W = rho' of CauchyLoss per observation
+ * under LFBA_CFG_ROBUST (the Corrector's scaling of J, rho'' < 0), else 1; distance-constraint rows included. Not
+ * multiplied by sigma2. Rows and columns that are exactly 0: camera entries beyond the live NC, camera[0] and camera[2] in
+ * recalibration (SubsetManifold), the gauge frame, frames without observations, all poses without REFINE_POSES.
+ * Gauge: with points refined, rigid motion of the scene (and without a distance constraint its scale) is free; the
+ * first frame with observations is held fixed. Without constraints the scale trades against bL0 and B and the call
+ * returns LFBA_INVALID_ARGUMENT, except in recalibration, where the constant fL and B fix the scale (DESIGN.md 10).
+ * LFBA_FAILURE when an undamped point block Hpp or a pivot of the undamped reduced system is not positive. */
+#define LFBA_GAUGE_NONE 0        /* points not refined: the reduced system is regular as it stands */
+#define LFBA_GAUGE_FIRST_FRAME 1 /* points refined (+ constraints or recalibration): pose of gauge_frame held fixed */
+typedef struct lfba_covariance_info {
+  int32_t gauge, gauge_frame;  /* gauge_frame = first frame with observations, -1 for LFBA_GAUGE_NONE */
+  int32_t n_reduced;           /* size of the system that was inverted */
+  int32_t reserved_i;
+  int64_t num_residuals;       /* 2N + K */
+  int64_t num_free_parameters; /* live camera + poses of observed frames + active points, minus the gauge */
+  double cost;                 /* 0.5 sum rho at the parameters */
+  double sigma2;               /* 2 cost / (num_residuals - num_free_parameters); 0 when that is not positive */
+  double gpu_ms;               /* device time of the call (CUDA events): evaluation, assembly, factorisation, inversion */
+  double selinv_ms;            /* of which the selected inversion and the read-out of the blocks */
+  double reserved[2];
+} lfba_covariance_info;
+
+/* Covariance blocks at the parameters lfba_solver_get_parameters returns. cov_camera17: 17x17 row-major; cov_poses:
+ * F x 6 x 6. Either may be NULL. Single-shard sessions only. The session is left as it was: a following
+ * lfba_solver_run produces the same iterations. */
+int lfba_solver_covariance(lfba_solver* s, double* cov_camera17, double* cov_poses, lfba_covariance_info* info);
+/* One-shot form for the drop-in caller of lfba_solve (it has no session), built like lfba_eval. */
+int lfba_covariance(const lfba_problem* pb, const lfba_options* opt, const double* camera17, const double* views6F,
+                    const double* points3P, double* cov_camera17, double* cov_poses, lfba_covariance_info* info);
+
 /* Measures the device's FP64 FMA throughput (TFLOP/s) with a dependent-chain-free DFMA kernel. */
 int lfba_measure_fp64_peak(int device, double* tflops);
 void lfba_solver_destroy(lfba_solver* s);

@@ -22,7 +22,8 @@ _lib = None
 _EXPORTS = ["lfba_version", "lfba_last_error", "lfba_status_string", "lfba_options_init", "lfba_device_count", "lfba_trim_cache",
             "lfba_solve", "lfba_eval", "lfba_comm_unique_id", "lfba_comm_create", "lfba_comm_destroy", "lfba_solver_create", "lfba_solver_set_parameters",
             "lfba_solver_get_parameters", "lfba_solver_run", "lfba_solver_time_eval", "lfba_solver_track_blocks",
-            "lfba_measure_fp64_peak", "lfba_solver_destroy", "lfba_project_to_raw", "lfba_epipolar_web", "lfba_init_plenoptic"]
+            "lfba_measure_fp64_peak", "lfba_solver_destroy", "lfba_project_to_raw", "lfba_epipolar_web", "lfba_init_plenoptic",
+            "lfba_solver_covariance", "lfba_covariance"]
 
 
 def load():
@@ -66,6 +67,9 @@ def load():
     L.lfba_epipolar_web.argtypes = [C.c_float, C.c_float, C.c_int32, ip, ip, dp, ip]
     L.lfba_init_plenoptic.argtypes = [C.c_double, C.c_double, C.c_int64, dp, ip, ip, C.c_int32, dp, C.c_int32, dp, dp, dp, dp,
                                       C.c_int32]
+    L.lfba_solver_covariance.argtypes = [C.c_void_p, dp, dp, C.POINTER(capi.CovarianceInfo)]
+    L.lfba_covariance.argtypes = [C.POINTER(capi.Problem), C.POINTER(capi.Options), dp, dp, dp, dp, dp,
+                                  C.POINTER(capi.CovarianceInfo)]
     _lib = L
     return L
 
@@ -146,6 +150,32 @@ def evaluate(pa: capi.ProblemArrays, camera, views, points, jacobians=True, opti
     return {"residuals": res.reshape(n, 2), "jac_camera": jc, "jac_view": jv, "jac_point": jp, "cost": cost.value,
             "stats": {"std_x": st.std_x, "std_y": st.std_y, "mae_x": st.mae_x, "mae_y": st.mae_y,
                       "num_points": st.num_points, "num_inliers": st.num_inliers}}
+
+
+def _covariance_result(cam, poses, info: capi.CovarianceInfo) -> dict:
+    inf = {f: getattr(info, f) for f, _ in capi.CovarianceInfo._fields_ if not f.startswith("reserved")}
+    s2 = info.sigma2
+    return {"camera": cam, "poses": poses, "info": inf,
+            "std_camera": np.sqrt(s2 * np.diag(cam)),
+            "std_poses": np.sqrt(s2 * np.diagonal(poses, axis1=1, axis2=2))}
+
+
+def covariance(pa: capi.ProblemArrays, camera, views, points, options: capi.Options | None = None) -> dict:
+    """lfba_covariance: covariance blocks of (J^T W J)^-1 of camera and poses at the given parameters (ceres::Covariance
+    semantics, not multiplied by sigma2). Returns {"camera": 17x17, "poses": Fx6x6, "info": {...}, "std_camera": 17,
+    "std_poses": Fx6}; the standard deviations are scaled by info["sigma2"]."""
+    L = load()
+    cam = np.ascontiguousarray(camera, np.float64)
+    vw = np.ascontiguousarray(views, np.float64)
+    pt = np.ascontiguousarray(points, np.float64)
+    cc = np.zeros((17, 17))
+    cp = np.zeros((pa.n_frames, 6, 6))
+    info = capi.CovarianceInfo()
+    o = options if options is not None else default_options()
+    p = pa.as_struct()
+    _check(L.lfba_covariance(C.byref(p), C.byref(o), capi._dp(cam), capi._dp(vw), capi._dp(pt), capi._dp(cc),
+                             capi._dp(cp), C.byref(info)), "lfba_covariance")
+    return _covariance_result(cc, cp, info)
 
 
 def project_to_raw(grid: "capi.LensGrid", feat_x, feat_y, vdepth, frame_idx=None, point_idx=None, device=-1):
@@ -300,6 +330,16 @@ class DeviceSolver:
         _check(self._L.lfba_solver_track_blocks(self._h, C.byref(n), C.byref(rs), capi._dp(rec), capi._dp(camsum),
                                                 capi._ip(tp), capi._ip(tf)), "lfba_solver_track_blocks")
         return {"rec": rec, "camsum": camsum, "trk_point": tp, "trk_frame": tf, "rec_stride": RS}
+
+    def covariance(self) -> dict:
+        """lfba_solver_covariance: covariance blocks of camera and poses at the parameters get_parameters() returns;
+        same result as the module-level covariance() there. The session is left as it was."""
+        cc = np.zeros((17, 17))
+        cp = np.zeros((self.pa.n_frames, 6, 6))
+        info = capi.CovarianceInfo()
+        _check(self._L.lfba_solver_covariance(self._h, capi._dp(cc), capi._dp(cp), C.byref(info)),
+               "lfba_solver_covariance")
+        return _covariance_result(cc, cp, info)
 
     def close(self):
         if self._h:

@@ -98,6 +98,16 @@ class ReprojStats(C.Structure):
                 ("num_points", C.c_int64), ("num_inliers", C.c_int64)]
 
 
+GAUGE_NONE, GAUGE_FIRST_FRAME = 0, 1
+
+
+class CovarianceInfo(C.Structure):
+    _fields_ = [("gauge", C.c_int32), ("gauge_frame", C.c_int32), ("n_reduced", C.c_int32), ("reserved_i", C.c_int32),
+                ("num_residuals", C.c_int64), ("num_free_parameters", C.c_int64),
+                ("cost", C.c_double), ("sigma2", C.c_double), ("gpu_ms", C.c_double), ("selinv_ms", C.c_double),
+                ("reserved", C.c_double * 2)]
+
+
 class Comm(C.Structure):
     _fields_ = [("rank", C.c_int32), ("nranks", C.c_int32), ("nccl_unique_id", C.c_char * 128), ("handle", C.c_void_p)]
 

@@ -351,6 +351,10 @@ void launch_chol_banded(const Dev& d, int bw, int nb, size_t smem, cudaStream_t 
 
 int launch_reduced_solve(const Dev& d, int n_tiles, const int* d_tile_first, int bw, cudaStream_t s, PartPlan* plan) {
   if (part_plan_active(plan)) return launch_part_solve(d, plan, s);
+  return launch_chol_inplace(d, n_tiles, d_tile_first, bw, s);
+}
+
+int launch_chol_inplace(const Dev& d, int n_tiles, const int* d_tile_first, int bw, cudaStream_t s) {
   const int nb = d.n - d.np6 + 1;
   const size_t bsm = banded_smem_bytes(d, bw, nb);
   if (bsm > 0) {

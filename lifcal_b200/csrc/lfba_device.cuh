@@ -152,6 +152,8 @@ struct Dev {
   uint32_t config;
   int recalib, refine_poses, refine_points;
   int debug;                // LFBA_DEBUG set: the control kernel prints its line-search decisions
+  int undamped;             // covariance: assemble J^T W J itself (no LM damping; k_finalize keeps no iteration row)
+  int gauge_frame;          // covariance: frame whose pose is held fixed (identity rows in S), -1 = none
   double spx, spy, scale;
   Options opt;
   // observations (sorted by point, frame)

@@ -661,7 +661,7 @@ __global__ void __launch_bounds__(128) k_points(Dev d) {
     double dmp[3];
     for (int j = 0; j < 3; ++j) {
       const double s2 = ps[j] * ps[j];
-      dmp[j] = fmin(fmax(s2 * hd[j], d.opt.min_diag), d.opt.max_diag) / (mu * s2);
+      dmp[j] = d.undamped ? 0.0 : fmin(fmax(s2 * hd[j], d.opt.min_diag), d.opt.max_diag) / (mu * s2);
     }
     const double Hd[6] = {H[0] + dmp[0], H[1], H[2], H[3] + dmp[1], H[4], H[5] + dmp[2]};
     double Hi[6];
@@ -1118,6 +1118,19 @@ __global__ void __launch_bounds__(1024) k_add_camera(Dev d) {
 __global__ void __launch_bounds__(1024) k_finalize(Dev d) {
   LmState* st = d.st;
   if (linear_phase_idle(st)) return;
+  if (d.undamped) {
+    // covariance: S stays the Gauss-Newton matrix (the min_lm_diagonal clamp would damp even an infinite radius); the
+    // pose rows and columns of the gauge frame and of frames without observations become identity
+    if (threadIdx.x == 0) st->solve_ok = d.sys_scalars[SS_PTFAIL] > 0.0 ? 0 : 1;
+    auto fixed = [&](int r) { return r < d.np6 && (r / 6 == d.gauge_frame || !d.frm_active[r / 6]); };
+    const int lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+    for (int r = threadIdx.x >> 5; r < d.n; r += nw) {
+      const bool fr = fixed(r);
+      for (int c = d.row_c0[r] + lane; c <= r; c += 32)
+        if (fr || fixed(c)) *S_at(d, r, c) = r == c ? 1.0 : 0.0;
+    }
+    return;
+  }
   const Options& o = d.opt;
   __shared__ double sg2[32], sgm[32];
   const bool first = st->first != 0;

@@ -34,6 +34,15 @@ bool part_plan_active(const PartPlan* p);
 int launch_part_solve(const Dev& d, PartPlan* p, cudaStream_t s);
 int launch_reduced_solve(const Dev& d, int n_tiles, const int* d_tile_first /*[n_tiles] first nonzero tile col*/,
                          int bandwidth_frames, cudaStream_t s, PartPlan* plan);
+// The in-place factorisations only (banded one-CTA kernel when it fits, else the tiled one): L is left in d.S, in the
+// skyline layout, unpermuted. Returns the number of kernels launched.
+int launch_chol_inplace(const Dev& d, int n_tiles, const int* d_tile_first, int bandwidth_frames, cudaStream_t s);
+
+// ---- lfba_cov.cu: covariance from the factorised reduced system ----
+void prepare_cov_kernels();
+// Selected inversion of L L^T (L in d.S) over the skyline envelope into Z (same layout, S_len doubles), then the
+// 17 x 17 camera block and the F x 6 x 6 pose blocks into out[289 + 36 F]. Returns the number of kernels launched.
+int launch_covariance(const Dev& d, double* Z, double* out, cudaStream_t s);
 
 // ---- lfba_eval.cu: eval-only kernel (residuals + Jacobians materialised in Ceres' block layout) ----
 struct EvalOut {

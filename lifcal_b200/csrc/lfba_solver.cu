@@ -446,6 +446,7 @@ struct Solver {
     ev_made = true;
     prepare_device_kernels();
     prepare_eval_kernels();
+    prepare_cov_kernels();
     dbg_phase("events + kernel attributes");
     part_plan = part_plan_create(d, band_frames, stream);
     LFBA_CUDA(cudaStreamSynchronize(stream));
@@ -537,6 +538,97 @@ struct Solver {
     launches += launch_steps(d, stream);
     launches += launch_ls_apply(d, stream);
     mark(LFBA_T_POINTSTEP);
+  }
+
+  // ---- covariance of camera and poses at the accepted parameters (lfba_solver_covariance) ----
+  // One evaluation pass and the Schur assembly of the undamped J^T W J there, the in-place Cholesky, the selected
+  // inversion. It runs on the round's work buffers with a fresh device LmState; the host's h_state and the caller's
+  // parameters (camera0 ...) are not touched, and run() rebuilds everything else from them.
+  void covariance(double* cov_cam, double* cov_poses, lfba_covariance_info* info) {
+    LFBA_CUDA(cudaSetDevice(device));
+    alloc_stream() = stream;
+    if (!camera0.p) throw CudaError("lfba_solver_covariance before lfba_solver_set_parameters", LFBA_INVALID_ARGUMENT);
+    const bool recalib = calib_type == LFBA_RECALIBRATION;
+    // with points refined, rigid motion + scale are free; a distance constraint (or recalibration's constant fL and B)
+    // fixes the scale, and holding one frame's pose then removes the rest (DESIGN.md section 10)
+    if (d.refine_points && K == 0 && !recalib)
+      throw CudaError("covariance: points are refined without a distance constraint, so the scale gauge (scene scale "
+                      "against bL0 and B) leaves the covariance undefined", LFBA_INVALID_ARGUMENT);
+    int gf = -1;
+    if (d.refine_points)
+      for (int f = 0; f < ix.F && gf < 0; ++f)
+        if (h_fa[f]) gf = f;
+    Dev dc = d;
+    dc.undamped = 1;
+    dc.gauge_frame = gf;
+    const int F = ix.F;
+    cudaEvent_t e0, e1, e2;
+    LFBA_CUDA(cudaEventCreate(&e0));
+    LFBA_CUDA(cudaEventCreate(&e1));
+    LFBA_CUDA(cudaEventCreate(&e2));
+    LFBA_CUDA(cudaEventRecord(e0, stream));
+    LmState init;
+    std::memset(&init, 0, sizeof(init));
+    init.cur = 1 - h_state.cur;  // the accepted parameters enter as the candidate of iteration zero
+    init.solve_ok = 1;
+    LFBA_CUDA(cudaMemcpyAsync(st.p, &init, sizeof(LmState), cudaMemcpyHostToDevice, stream));
+    launch_tables(dc, stream);
+    launches += launch_eval(dc, lanes, stream);
+    launch_reduce_eval(dc, stream);
+    launch_control_accept(dc, stream);  // iteration zero: the candidate becomes the accepted state, its cost x_cost
+    LFBA_CUDA(cudaMemsetAsync(redbuf.p, 0, red_len * sizeof(double), stream));
+    launches += 3 + launch_assembly(dc, frame_splits, stream);
+    launch_finalize(dc, stream);
+    launches += 1 + launch_chol_inplace(dc, n_tiles, tile_first.p, band_frames, stream);
+    LFBA_CUDA(cudaEventRecord(e1, stream));
+    DevBuf<double> Z(S_len), out((size_t)289 + 36 * (size_t)F);
+    launches += launch_covariance(dc, Z.p, out.p, stream);
+    LFBA_CUDA(cudaEventRecord(e2, stream));
+    std::vector<double> h_out((size_t)289 + 36 * (size_t)F);
+    out.download(h_out.data(), h_out.size(), stream);
+    LmState hs;
+    double ptfail = 0.0;
+    LFBA_CUDA(cudaMemcpyAsync(&hs, st.p, sizeof(LmState), cudaMemcpyDeviceToHost, stream));
+    LFBA_CUDA(cudaMemcpyAsync(&ptfail, d.sys_scalars + SS_PTFAIL, sizeof(double), cudaMemcpyDeviceToHost, stream));
+    std::vector<int32_t> h_pa;
+    if (d.refine_points) {
+      h_pa.resize((size_t)ix.P);
+      pt_active.download(h_pa.data(), (size_t)ix.P, stream);
+    }
+    LFBA_CUDA(cudaStreamSynchronize(stream));
+    LFBA_CUDA(cudaGetLastError());
+    float ms_all = 0.f, ms_inv = 0.f;
+    cudaEventElapsedTime(&ms_all, e0, e2);
+    cudaEventElapsedTime(&ms_inv, e1, e2);
+    cudaEventDestroy(e0);
+    cudaEventDestroy(e1);
+    cudaEventDestroy(e2);
+    if (ptfail > 0.0)
+      throw CudaError("covariance: an undamped point block Hpp is not positive definite (a point is not determined by "
+                      "its observations)", LFBA_FAILURE);
+    if (!hs.solve_ok)
+      throw CudaError("covariance: a pivot of the undamped reduced system is not positive (J^T W J is singular at "
+                      "these parameters)", LFBA_FAILURE);
+    if (cov_cam) std::memcpy(cov_cam, h_out.data(), 289 * sizeof(double));
+    if (cov_poses) std::memcpy(cov_poses, h_out.data() + 289, (size_t)36 * F * sizeof(double));
+    if (info) {
+      std::memset(info, 0, sizeof(*info));
+      info->gauge = gf >= 0 ? LFBA_GAUGE_FIRST_FRAME : LFBA_GAUGE_NONE;
+      info->gauge_frame = gf;
+      info->n_reduced = d.n;
+      info->num_residuals = 2 * n_obs_global + K;
+      int64_t np = d.n_cam_red;
+      if (d.refine_poses)
+        for (int f = 0; f < F; ++f) np += h_fa[f] ? 6 : 0;
+      for (int32_t a : h_pa) np += a ? 3 : 0;
+      if (gf >= 0) np -= 6;
+      info->num_free_parameters = np;
+      info->cost = hs.x_cost;
+      const int64_t dof = info->num_residuals - np;
+      info->sigma2 = dof > 0 ? 2.0 * hs.x_cost / (double)dof : 0.0;
+      info->gpu_ms = ms_all;
+      info->selinv_ms = ms_inv;
+    }
   }
 };
 
@@ -1061,6 +1153,17 @@ int lfba_solver_track_blocks(lfba_solver* h, int64_t* n_tracks, int32_t* rec_str
   });
 }
 
+int lfba_solver_covariance(lfba_solver* h, double* cov_camera17, double* cov_poses, lfba_covariance_info* info) {
+  if (!h) return LFBA_INVALID_ARGUMENT;
+  return guarded([&] {
+    if (h->g.emulated() || h->g.nranks > 1)
+      throw CudaError("lfba_solver_covariance: single-shard sessions only (the reduced system of a sharded session is "
+                      "summed over its shards)", LFBA_INVALID_ARGUMENT);
+    h->g.s0().covariance(cov_camera17, cov_poses, info);
+    return (int)LFBA_OK;
+  });
+}
+
 int lfba_measure_fp64_peak(int device, double* tflops) {
   if (!tflops) return LFBA_INVALID_ARGUMENT;
   return guarded([&] {
@@ -1120,6 +1223,21 @@ int lfba_eval(const lfba_problem* pb, const lfba_options* opt_in, const double* 
       stats->num_points = N;
       stats->num_inliers = (int64_t)(hs[4] + 0.5);
     }
+    return (int)LFBA_OK;
+  });
+}
+
+int lfba_covariance(const lfba_problem* pb, const lfba_options* opt_in, const double* cam, const double* views,
+                    const double* points, double* cov_camera17, double* cov_poses, lfba_covariance_info* info) {
+  if (!pb || !cam || !views || !points) return LFBA_INVALID_ARGUMENT;
+  lfba_options o;
+  if (opt_in) o = *opt_in; else lfba_options_init(&o);
+  o.emulate_shards = 0;
+  return guarded([&] {
+    Group g;
+    g.create(*pb, o, nullptr);
+    g.set_parameters(cam, views, points);
+    g.s0().covariance(cov_camera17, cov_poses, info);
     return (int)LFBA_OK;
   });
 }
