@@ -328,7 +328,8 @@ typedef struct lfba_covariance_info {
   double sigma2;               /* 2 cost / (num_residuals - num_free_parameters); 0 when that is not positive */
   double gpu_ms;               /* device time of the call (CUDA events): evaluation, assembly, factorisation, inversion */
   double selinv_ms;            /* of which the selected inversion and the read-out of the blocks */
-  double reserved[2];
+  double points_ms;            /* device time of the per-point blocks (not part of gpu_ms); 0 when they were not asked for */
+  double reserved[1];
 } lfba_covariance_info;
 
 /* Covariance blocks at the parameters lfba_solver_get_parameters returns. cov_camera17: 17x17 row-major; cov_poses:
@@ -338,6 +339,19 @@ int lfba_solver_covariance(lfba_solver* s, double* cov_camera17, double* cov_pos
 /* One-shot form for the drop-in caller of lfba_solve (it has no session), built like lfba_eval. */
 int lfba_covariance(const lfba_problem* pb, const lfba_options* opt, const double* camera17, const double* views6F,
                     const double* points3P, double* cov_camera17, double* cov_poses, lfba_covariance_info* info);
+/* The same, plus the 3 x 3 covariance block of every point: cov_points is P x 3 x 3 row-major (must not be NULL), each
+ * block exactly symmetric (ceres::Covariance::GetCovarianceBlock(point, point)). Camera, poses and info other than
+ * points_ms are those lfba_solver_covariance / lfba_covariance return, bit for bit. Blocks that are exactly 0: points
+ * without observations and constraints, and every point without REFINE_POINTS (constant blocks, status LFBA_OK). With
+ * points refined, the blocks are relative to the gauge: the first frame with observations held fixed, so a point's
+ * uncertainty is the uncertainty of its position in that frame's pose, not in an absolute world frame. Points coupled
+ * by a distance constraint get their block of the reduced system's inverse. On a non-OK status cov_points may have been
+ * overwritten (with zeros). */
+int lfba_solver_covariance_points(lfba_solver* s, double* cov_camera17, double* cov_poses, double* cov_points,
+                                  lfba_covariance_info* info);
+int lfba_covariance_points(const lfba_problem* pb, const lfba_options* opt, const double* camera17, const double* views6F,
+                           const double* points3P, double* cov_camera17, double* cov_poses, double* cov_points,
+                           lfba_covariance_info* info);
 
 /* Measures the device's FP64 FMA throughput (TFLOP/s) with a dependent-chain-free DFMA kernel. */
 int lfba_measure_fp64_peak(int device, double* tflops);

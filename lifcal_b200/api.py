@@ -23,7 +23,7 @@ _EXPORTS = ["lfba_version", "lfba_last_error", "lfba_status_string", "lfba_optio
             "lfba_solve", "lfba_eval", "lfba_comm_unique_id", "lfba_comm_create", "lfba_comm_destroy", "lfba_solver_create", "lfba_solver_set_parameters",
             "lfba_solver_get_parameters", "lfba_solver_run", "lfba_solver_time_eval", "lfba_solver_track_blocks",
             "lfba_measure_fp64_peak", "lfba_solver_destroy", "lfba_project_to_raw", "lfba_epipolar_web", "lfba_init_plenoptic",
-            "lfba_solver_covariance", "lfba_covariance"]
+            "lfba_solver_covariance", "lfba_covariance", "lfba_solver_covariance_points", "lfba_covariance_points"]
 
 
 def load():
@@ -70,6 +70,9 @@ def load():
     L.lfba_solver_covariance.argtypes = [C.c_void_p, dp, dp, C.POINTER(capi.CovarianceInfo)]
     L.lfba_covariance.argtypes = [C.POINTER(capi.Problem), C.POINTER(capi.Options), dp, dp, dp, dp, dp,
                                   C.POINTER(capi.CovarianceInfo)]
+    L.lfba_solver_covariance_points.argtypes = [C.c_void_p, dp, dp, dp, C.POINTER(capi.CovarianceInfo)]
+    L.lfba_covariance_points.argtypes = [C.POINTER(capi.Problem), C.POINTER(capi.Options), dp, dp, dp, dp, dp, dp,
+                                         C.POINTER(capi.CovarianceInfo)]
     _lib = L
     return L
 
@@ -152,18 +155,24 @@ def evaluate(pa: capi.ProblemArrays, camera, views, points, jacobians=True, opti
                       "num_points": st.num_points, "num_inliers": st.num_inliers}}
 
 
-def _covariance_result(cam, poses, info: capi.CovarianceInfo) -> dict:
+def _covariance_result(cam, poses, info: capi.CovarianceInfo, points=None) -> dict:
     inf = {f: getattr(info, f) for f, _ in capi.CovarianceInfo._fields_ if not f.startswith("reserved")}
     s2 = info.sigma2
-    return {"camera": cam, "poses": poses, "info": inf,
-            "std_camera": np.sqrt(s2 * np.diag(cam)),
-            "std_poses": np.sqrt(s2 * np.diagonal(poses, axis1=1, axis2=2))}
+    r = {"camera": cam, "poses": poses, "info": inf,
+         "std_camera": np.sqrt(s2 * np.diag(cam)),
+         "std_poses": np.sqrt(s2 * np.diagonal(poses, axis1=1, axis2=2))}
+    if points is not None:
+        r["points"] = points
+        r["std_points"] = np.sqrt(s2 * np.diagonal(points, axis1=1, axis2=2))
+    return r
 
 
-def covariance(pa: capi.ProblemArrays, camera, views, points, options: capi.Options | None = None) -> dict:
+def covariance(pa: capi.ProblemArrays, camera, views, points, options: capi.Options | None = None,
+               with_points: bool = False) -> dict:
     """lfba_covariance: covariance blocks of (J^T W J)^-1 of camera and poses at the given parameters (ceres::Covariance
     semantics, not multiplied by sigma2). Returns {"camera": 17x17, "poses": Fx6x6, "info": {...}, "std_camera": 17,
-    "std_poses": Fx6}; the standard deviations are scaled by info["sigma2"]."""
+    "std_poses": Fx6}; the standard deviations are scaled by info["sigma2"]. with_points: lfba_covariance_points, which
+    also returns "points" (P x 3 x 3, relative to the gauge frame) and "std_points" (P x 3)."""
     L = load()
     cam = np.ascontiguousarray(camera, np.float64)
     vw = np.ascontiguousarray(views, np.float64)
@@ -173,9 +182,14 @@ def covariance(pa: capi.ProblemArrays, camera, views, points, options: capi.Opti
     info = capi.CovarianceInfo()
     o = options if options is not None else default_options()
     p = pa.as_struct()
-    _check(L.lfba_covariance(C.byref(p), C.byref(o), capi._dp(cam), capi._dp(vw), capi._dp(pt), capi._dp(cc),
-                             capi._dp(cp), C.byref(info)), "lfba_covariance")
-    return _covariance_result(cc, cp, info)
+    if not with_points:
+        _check(L.lfba_covariance(C.byref(p), C.byref(o), capi._dp(cam), capi._dp(vw), capi._dp(pt), capi._dp(cc),
+                                 capi._dp(cp), C.byref(info)), "lfba_covariance")
+        return _covariance_result(cc, cp, info)
+    cq = np.zeros((pa.n_points, 3, 3))
+    _check(L.lfba_covariance_points(C.byref(p), C.byref(o), capi._dp(cam), capi._dp(vw), capi._dp(pt), capi._dp(cc),
+                                    capi._dp(cp), capi._dp(cq), C.byref(info)), "lfba_covariance_points")
+    return _covariance_result(cc, cp, info, cq)
 
 
 def project_to_raw(grid: "capi.LensGrid", feat_x, feat_y, vdepth, frame_idx=None, point_idx=None, device=-1):
@@ -331,15 +345,21 @@ class DeviceSolver:
                                                 capi._ip(tp), capi._ip(tf)), "lfba_solver_track_blocks")
         return {"rec": rec, "camsum": camsum, "trk_point": tp, "trk_frame": tf, "rec_stride": RS}
 
-    def covariance(self) -> dict:
+    def covariance(self, with_points: bool = False) -> dict:
         """lfba_solver_covariance: covariance blocks of camera and poses at the parameters get_parameters() returns;
-        same result as the module-level covariance() there. The session is left as it was."""
+        same result as the module-level covariance() there. The session is left as it was. with_points:
+        lfba_solver_covariance_points, which also returns "points" (P x 3 x 3) and "std_points" (P x 3)."""
         cc = np.zeros((17, 17))
         cp = np.zeros((self.pa.n_frames, 6, 6))
         info = capi.CovarianceInfo()
-        _check(self._L.lfba_solver_covariance(self._h, capi._dp(cc), capi._dp(cp), C.byref(info)),
-               "lfba_solver_covariance")
-        return _covariance_result(cc, cp, info)
+        if not with_points:
+            _check(self._L.lfba_solver_covariance(self._h, capi._dp(cc), capi._dp(cp), C.byref(info)),
+                   "lfba_solver_covariance")
+            return _covariance_result(cc, cp, info)
+        cq = np.zeros((self.pa.n_points, 3, 3))
+        _check(self._L.lfba_solver_covariance_points(self._h, capi._dp(cc), capi._dp(cp), capi._dp(cq), C.byref(info)),
+               "lfba_solver_covariance_points")
+        return _covariance_result(cc, cp, info, cq)
 
     def close(self):
         if self._h:

@@ -105,7 +105,7 @@ class CovarianceInfo(C.Structure):
     _fields_ = [("gauge", C.c_int32), ("gauge_frame", C.c_int32), ("n_reduced", C.c_int32), ("reserved_i", C.c_int32),
                 ("num_residuals", C.c_int64), ("num_free_parameters", C.c_int64),
                 ("cost", C.c_double), ("sigma2", C.c_double), ("gpu_ms", C.c_double), ("selinv_ms", C.c_double),
-                ("reserved", C.c_double * 2)]
+                ("points_ms", C.c_double), ("reserved", C.c_double * 1)]
 
 
 class Comm(C.Structure):

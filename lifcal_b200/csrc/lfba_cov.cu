@@ -136,6 +136,160 @@ __global__ void k_cov_gather(Dev d, const double* __restrict__ Z, double* __rest
   }
 }
 
+// Per-point 3 x 3 blocks. An eliminated point p (pdata written by the undamped k_points) has, with Hi = Hpp^-1 and u the
+// point's n x 3 coupling column of J^T W J (V_t^T of its tracks in pose rows, Hcp in camera rows),
+//     Sigma_pp = Hi + Hi Q Hi,   Q = u^T Z u = sum_{a,b} V_a^T Z[f_a, f_b] V_b + (M + M^T) + Hcp^T Z[cam, cam] Hcp,
+//     M = sum_a V_a^T Z[f_a, cam] Hcp
+// (block inverse of [[S, u], [u^T, Hpp]]). Q is symmetric, so it is its own symmetric part sym(X) = (X + X^T) / 2, and
+// sym(V_a^T Z_ab V_b) = sym(V_b^T Z_ba V_a): with one track per (point, frame),
+//     Q = sym( sum_a V_a^T y_a ) + Hcp^T Z[cam, cam] Hcp,   y_a = Z[f_a, f_a] V_a + 2 (sum_{f_b < f_a} Z[f_a, f_b] V_b + Z[f_a, cam] Hcp)
+// reads only lower blocks of Z (row f_a, columns 6 f_b .. contiguous) and does half the pairs, 108 FMA each. Tracks in
+// the gauge frame are skipped: that pose is not a parameter, and Z holds identity on its rows. Frames of one point are at
+// most `band` apart, so every Z[f_a, f_b] lies in the envelope. A coupled point's block is its diagonal block of Z. One
+// thread per point.
+template <int NC>
+__global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restrict__ Z, double* __restrict__ out) {
+  const SkyMap sky{d.band, d.np6};
+  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < d.P; p += gridDim.x * blockDim.x) {
+    double Sg[6] = {0, 0, 0, 0, 0, 0};  // lower triangle: 00 10 11 20 21 22
+    const int cp = d.refine_points && d.st->solve_ok && d.pt_active[p] ? d.pt_coupled[p] : -2;
+    if (cp >= 0) {
+      const int r0 = d.np6 + 3 * cp;
+#pragma unroll
+      for (int i = 0, h = 0; i < 3; ++i)
+#pragma unroll
+        for (int j = 0; j <= i; ++j, ++h) Sg[h] = Z[sky_off(sky, r0 + i, r0 + j)];
+    } else if (cp == -1) {
+      const double* __restrict__ pd = d.pdata + (size_t)p * kPointStride;
+      const double* __restrict__ Hc = pd + 12;  // Hcp[3 c + j]; columns with cam_red[c] < 0 are skipped
+      double Q[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+      if (d.refine_poses) {
+        const int t0 = d.pt_trk_begin[p], t1 = d.pt_trk_begin[p + 1];
+        for (int a = t0; a < t1; ++a) {
+          const int fa = d.trk_frame[a];
+          if (fa == d.gauge_frame) continue;
+          const long long za = sky.row(fa, 0) - sky.c0(fa);  // + offset of row i + column: entry (6 fa + i, column)
+          const int len0 = 6 * fa - sky.c0(fa) + 1;
+          auto zrow = [&](int i) { return za + (long long)i * len0 + (i * (i - 1)) / 2; };
+          double y[18];
+#pragma unroll
+          for (int k = 0; k < 18; ++k) y[k] = 0.0;
+          // pose-camera (camera rows are border rows: Z[r, 6 fa + i] is contiguous in i)
+#pragma unroll
+          for (int c = 0; c < NC; ++c) {
+            const int r = d.cam_red[c];
+            if (r < 0) continue;
+            const double* zr = Z + sky.border_row(r - d.np6) + 6 * fa;
+            const double h0 = Hc[3 * c], h1 = Hc[3 * c + 1], h2 = Hc[3 * c + 2];
+#pragma unroll
+            for (int i = 0; i < 6; ++i) {
+              const double z = zr[i];
+              y[3 * i] += z * h0;
+              y[3 * i + 1] += z * h1;
+              y[3 * i + 2] += z * h2;
+            }
+          }
+          // pose-pose, frames before fa
+          for (int b = t0; b < t1; ++b) {
+            const int fb = d.trk_frame[b];
+            if (fb >= fa || fb == d.gauge_frame) continue;
+            double Vb[18];
+            const double* Vp = d.vw + (size_t)b * kVWStride;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) ldg256(Vp + 4 * k, Vb + 4 * k);
+            const double2 v2 = __ldg(reinterpret_cast<const double2*>(Vp) + 8);
+            Vb[16] = v2.x;
+            Vb[17] = v2.y;
+#pragma unroll
+            for (int i = 0; i < 6; ++i) {
+              const double* zr = Z + zrow(i) + 6 * fb;
+#pragma unroll
+              for (int j = 0; j < 6; ++j) {
+                const double z = zr[j];
+#pragma unroll
+                for (int k = 0; k < 3; ++k) y[3 * i + k] += z * Vb[3 * j + k];
+              }
+            }
+          }
+          double Va[18];
+          {
+            const double* Vp = d.vw + (size_t)a * kVWStride;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) ldg256(Vp + 4 * k, Va + 4 * k);
+            const double2 v2 = __ldg(reinterpret_cast<const double2*>(Vp) + 8);
+            Va[16] = v2.x;
+            Va[17] = v2.y;
+          }
+#pragma unroll
+          for (int k = 0; k < 18; ++k) y[k] *= 2.0;
+          // diagonal block Z[fa, fa], read from its lower triangle
+#pragma unroll
+          for (int i = 0; i < 6; ++i)
+#pragma unroll
+            for (int j = 0; j < 6; ++j) {
+              const double z = i >= j ? Z[zrow(i) + 6 * fa + j] : Z[zrow(j) + 6 * fa + i];
+#pragma unroll
+              for (int k = 0; k < 3; ++k) y[3 * i + k] += z * Va[3 * j + k];
+            }
+#pragma unroll
+          for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int j = 0; j < 3; ++j) {
+              double m = 0.0;
+#pragma unroll
+              for (int k = 0; k < 6; ++k) m += Va[3 * k + i] * y[3 * k + j];
+              Q[3 * i + j] += m;
+            }
+        }
+      }
+      // camera-camera (the outer loop unrolled as well gives 255 registers and spills; rolled: 128, none)
+#pragma unroll 1
+      for (int c1 = 0; c1 < NC; ++c1) {
+        const int r1 = d.cam_red[c1];
+        if (r1 < 0) continue;
+        double y[3] = {0, 0, 0};
+#pragma unroll
+        for (int c2 = 0; c2 < NC; ++c2) {
+          const int r2 = d.cam_red[c2];
+          if (r2 < 0) continue;
+          const double z = sym_at(Z, sky, r1, r2);
+#pragma unroll
+          for (int j = 0; j < 3; ++j) y[j] += z * Hc[3 * c2 + j];
+        }
+#pragma unroll
+        for (int i = 0; i < 3; ++i)
+#pragma unroll
+          for (int j = 0; j < 3; ++j) Q[3 * i + j] += Hc[3 * c1 + i] * y[j];
+      }
+      // Sigma = Hi + Hi sym(Q) Hi
+      const double Hi[9] = {pd[0], pd[1], pd[2], pd[1], pd[3], pd[4], pd[2], pd[4], pd[5]};
+      double T[9];
+#pragma unroll
+      for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int j = 0; j < 3; ++j) {
+          double v = 0.0;
+#pragma unroll
+          for (int k = 0; k < 3; ++k) v += Hi[3 * i + k] * (0.5 * (Q[3 * k + j] + Q[3 * j + k]));
+          T[3 * i + j] = v;
+        }
+#pragma unroll
+      for (int i = 0, h = 0; i < 3; ++i)
+#pragma unroll
+        for (int j = 0; j <= i; ++j, ++h) {
+          double v = Hi[3 * i + j];
+#pragma unroll
+          for (int k = 0; k < 3; ++k) v += T[3 * i + k] * Hi[3 * k + j];
+          Sg[h] = v;
+        }
+    }
+    double* o = out + 9 * (size_t)p;
+    o[0] = Sg[0]; o[1] = Sg[1]; o[2] = Sg[3];
+    o[3] = Sg[1]; o[4] = Sg[2]; o[5] = Sg[4];
+    o[6] = Sg[3]; o[7] = Sg[4]; o[8] = Sg[5];
+  }
+}
+
 static size_t selinv_y_doubles(const Dev& d) { return 6 * (size_t)(6 * d.band + (d.n - d.np6) + 1); }
 
 void prepare_cov_kernels() {
@@ -151,6 +305,12 @@ int launch_covariance(const Dev& d, double* Z, double* out, cudaStream_t s) {
   const int total = 289 + 36 * d.F;
   k_cov_gather<<<(total + 255) / 256, 256, 0, s>>>(d, Z, out);
   return 2;
+}
+
+int launch_cov_points(const Dev& d, const double* Z, double* out, cudaStream_t s) {
+  if (d.P == 0) return 0;
+  LFBA_DISPATCH_NC(d.NC, (k_cov_points<NC><<<d.grid_pts, 128, 0, s>>>(d, Z, out)));
+  return 1;
 }
 
 }  // namespace lfba

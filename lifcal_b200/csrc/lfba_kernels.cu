@@ -1416,15 +1416,6 @@ __global__ void __launch_bounds__(128) k_init_norms(Dev d) {
 // ================================================================================================
 // launchers
 // ================================================================================================
-#define LFBA_DISPATCH_NC(NCV, CALL)   \
-  switch (NCV) {                      \
-    case 5: { constexpr int NC = 5; CALL; } break; \
-    case 6: { constexpr int NC = 6; CALL; } break; \
-    case 7: { constexpr int NC = 7; CALL; } break; \
-    case 8: { constexpr int NC = 8; CALL; } break; \
-    default: { constexpr int NC = 9; CALL; } break; \
-  }
-
 void prepare_eval_kernels() {
   prepare_rows_kernels();
   prepare_eval_only_kernels();

@@ -6,6 +6,16 @@
 
 namespace lfba {
 
+// CALL with `NC` a compile-time constant equal to the live camera parameter count NCV (5 .. 9)
+#define LFBA_DISPATCH_NC(NCV, CALL)   \
+  switch (NCV) {                      \
+    case 5: { constexpr int NC = 5; CALL; } break; \
+    case 6: { constexpr int NC = 6; CALL; } break; \
+    case 7: { constexpr int NC = 7; CALL; } break; \
+    case 8: { constexpr int NC = 8; CALL; } break; \
+    default: { constexpr int NC = 9; CALL; } break; \
+  }
+
 // ---- lfba_kernels.cu: one LM round ----
 void launch_init_norms(const Dev& d, cudaStream_t s);
 void launch_tables(const Dev& d, cudaStream_t s);
@@ -43,6 +53,9 @@ void prepare_cov_kernels();
 // Selected inversion of L L^T (L in d.S) over the skyline envelope into Z (same layout, S_len doubles), then the
 // 17 x 17 camera block and the F x 6 x 6 pose blocks into out[289 + 36 F]. Returns the number of kernels launched.
 int launch_covariance(const Dev& d, double* Z, double* out, cudaStream_t s);
+// After launch_covariance on the same stream: the 3 x 3 block of every point into out[9 P] (row-major, exactly
+// symmetric; zero for inactive points and when points are not refined). Returns the number of kernels launched.
+int launch_cov_points(const Dev& d, const double* Z, double* out, cudaStream_t s);
 
 // ---- lfba_eval.cu: eval-only kernel (residuals + Jacobians materialised in Ceres' block layout) ----
 struct EvalOut {

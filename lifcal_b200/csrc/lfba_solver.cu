@@ -543,8 +543,9 @@ struct Solver {
   // ---- covariance of camera and poses at the accepted parameters (lfba_solver_covariance) ----
   // One evaluation pass and the Schur assembly of the undamped J^T W J there, the in-place Cholesky, the selected
   // inversion. It runs on the round's work buffers with a fresh device LmState; the host's h_state and the caller's
-  // parameters (camera0 ...) are not touched, and run() rebuilds everything else from them.
-  void covariance(double* cov_cam, double* cov_poses, lfba_covariance_info* info) {
+  // parameters (camera0 ...) are not touched, and run() rebuilds everything else from them. With cov_points, the
+  // per-point blocks follow from the selected inverse and the point data of the same assembly (k_cov_points).
+  void covariance(double* cov_cam, double* cov_poses, double* cov_points, lfba_covariance_info* info) {
     LFBA_CUDA(cudaSetDevice(device));
     alloc_stream() = stream;
     if (!camera0.p) throw CudaError("lfba_solver_covariance before lfba_solver_set_parameters", LFBA_INVALID_ARGUMENT);
@@ -562,10 +563,11 @@ struct Solver {
     dc.undamped = 1;
     dc.gauge_frame = gf;
     const int F = ix.F;
-    cudaEvent_t e0, e1, e2;
+    cudaEvent_t e0, e1, e2, e3 = nullptr;
     LFBA_CUDA(cudaEventCreate(&e0));
     LFBA_CUDA(cudaEventCreate(&e1));
     LFBA_CUDA(cudaEventCreate(&e2));
+    if (cov_points) LFBA_CUDA(cudaEventCreate(&e3));
     LFBA_CUDA(cudaEventRecord(e0, stream));
     LmState init;
     std::memset(&init, 0, sizeof(init));
@@ -584,8 +586,15 @@ struct Solver {
     DevBuf<double> Z(S_len), out((size_t)289 + 36 * (size_t)F);
     launches += launch_covariance(dc, Z.p, out.p, stream);
     LFBA_CUDA(cudaEventRecord(e2, stream));
+    DevBuf<double> outp(cov_points ? (size_t)9 * ix.P : 0);
+    if (cov_points) {
+      launches += launch_cov_points(dc, Z.p, outp.p, stream);
+      LFBA_CUDA(cudaEventRecord(e3, stream));
+    }
     std::vector<double> h_out((size_t)289 + 36 * (size_t)F);
     out.download(h_out.data(), h_out.size(), stream);
+    if (cov_points && ix.P > 0)
+      LFBA_CUDA(cudaMemcpyAsync(cov_points, outp.p, (size_t)9 * ix.P * sizeof(double), cudaMemcpyDeviceToHost, stream));
     LmState hs;
     double ptfail = 0.0;
     LFBA_CUDA(cudaMemcpyAsync(&hs, st.p, sizeof(LmState), cudaMemcpyDeviceToHost, stream));
@@ -597,9 +606,13 @@ struct Solver {
     }
     LFBA_CUDA(cudaStreamSynchronize(stream));
     LFBA_CUDA(cudaGetLastError());
-    float ms_all = 0.f, ms_inv = 0.f;
+    float ms_all = 0.f, ms_inv = 0.f, ms_pts = 0.f;
     cudaEventElapsedTime(&ms_all, e0, e2);
     cudaEventElapsedTime(&ms_inv, e1, e2);
+    if (e3) {
+      cudaEventElapsedTime(&ms_pts, e2, e3);
+      cudaEventDestroy(e3);
+    }
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
     cudaEventDestroy(e2);
@@ -628,6 +641,7 @@ struct Solver {
       info->sigma2 = dof > 0 ? 2.0 * hs.x_cost / (double)dof : 0.0;
       info->gpu_ms = ms_all;
       info->selinv_ms = ms_inv;
+      info->points_ms = ms_pts;
     }
   }
 };
@@ -1159,7 +1173,19 @@ int lfba_solver_covariance(lfba_solver* h, double* cov_camera17, double* cov_pos
     if (h->g.emulated() || h->g.nranks > 1)
       throw CudaError("lfba_solver_covariance: single-shard sessions only (the reduced system of a sharded session is "
                       "summed over its shards)", LFBA_INVALID_ARGUMENT);
-    h->g.s0().covariance(cov_camera17, cov_poses, info);
+    h->g.s0().covariance(cov_camera17, cov_poses, nullptr, info);
+    return (int)LFBA_OK;
+  });
+}
+
+int lfba_solver_covariance_points(lfba_solver* h, double* cov_camera17, double* cov_poses, double* cov_points,
+                                  lfba_covariance_info* info) {
+  if (!h || !cov_points) return LFBA_INVALID_ARGUMENT;
+  return guarded([&] {
+    if (h->g.emulated() || h->g.nranks > 1)
+      throw CudaError("lfba_solver_covariance_points: single-shard sessions only (the reduced system of a sharded "
+                      "session is summed over its shards)", LFBA_INVALID_ARGUMENT);
+    h->g.s0().covariance(cov_camera17, cov_poses, cov_points, info);
     return (int)LFBA_OK;
   });
 }
@@ -1237,7 +1263,23 @@ int lfba_covariance(const lfba_problem* pb, const lfba_options* opt_in, const do
     Group g;
     g.create(*pb, o, nullptr);
     g.set_parameters(cam, views, points);
-    g.s0().covariance(cov_camera17, cov_poses, info);
+    g.s0().covariance(cov_camera17, cov_poses, nullptr, info);
+    return (int)LFBA_OK;
+  });
+}
+
+int lfba_covariance_points(const lfba_problem* pb, const lfba_options* opt_in, const double* cam, const double* views,
+                           const double* points, double* cov_camera17, double* cov_poses, double* cov_points,
+                           lfba_covariance_info* info) {
+  if (!pb || !cam || !views || !points || !cov_points) return LFBA_INVALID_ARGUMENT;
+  lfba_options o;
+  if (opt_in) o = *opt_in; else lfba_options_init(&o);
+  o.emulate_shards = 0;
+  return guarded([&] {
+    Group g;
+    g.create(*pb, o, nullptr);
+    g.set_parameters(cam, views, points);
+    g.s0().covariance(cov_camera17, cov_poses, cov_points, info);
     return (int)LFBA_OK;
   });
 }

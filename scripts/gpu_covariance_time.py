@@ -7,7 +7,11 @@ round); then the covariance at the solution is called `--reps` times after one w
 each call (it ends in a stream synchronise) and its CUDA-event times (whole call, selected inversion) are reported as
 median / min / max. The GPU's name, power limit and SM clocks are read in the same run.
 
-  python scripts/gpu_covariance_time.py [--reps 7] [--out covariance_time.json] [cfg3 cfg4]
+With --points, each repetition also calls covariance(with_points=True) right after the plain call on the same session,
+and reports its wall time, its device time of the per-point stage (points_ms) and, timed on its own with CUDA events
+through torch, the device-to-host copy of the 9 P doubles it returns into pageable host memory.
+
+  python scripts/gpu_covariance_time.py [--reps 7] [--points] [--out covariance_time.json] [cfg3 cfg4]
 """
 import argparse
 import json
@@ -16,6 +20,8 @@ import statistics
 import subprocess
 import sys
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -29,6 +35,23 @@ def gpu_state():
     return r.stdout.strip().splitlines()[0] if r.returncode == 0 and r.stdout.strip() else "unavailable"
 
 
+def d2h_copy_ms(n_doubles, reps):
+    """Device time of copying n doubles into pageable host memory (a fresh NumPy array, as the API returns)."""
+    import torch
+    src = torch.zeros(n_doubles, dtype=torch.float64, device="cuda")
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    out = []
+    for i in range(reps + 1):
+        dst = torch.from_numpy(np.zeros(n_doubles))
+        e0.record()
+        dst.copy_(src)
+        e1.record()
+        torch.cuda.synchronize()
+        if i:  # the first copy is a warm-up
+            out.append(e0.elapsed_time(e1))
+    return out
+
+
 def spread(v):
     return {"median": round(statistics.median(v), 4), "min": round(min(v), 4), "max": round(max(v), 4), "n": len(v)}
 
@@ -37,6 +60,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("workloads", nargs="*", default=["cfg3", "cfg4"])
     ap.add_argument("--reps", type=int, default=7)
+    ap.add_argument("--points", action="store_true", help="also time covariance(with_points=True)")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if api.device_count() < 1:
@@ -56,13 +80,22 @@ def main():
         rounds = s["kernel_calls"]["lens_pose_tables"]
         round_ms = sum(s["kernel_ms"].values()) / rounds
         ds.covariance()  # warm-up
+        if args.points:
+            ds.covariance(with_points=True)
         wall, dev, inv = [], [], []
+        pwall, pdev, pts = [], [], []
         for _ in range(args.reps):
             t = time.perf_counter()
             c = ds.covariance()
             wall.append(1e3 * (time.perf_counter() - t))
             dev.append(c["info"]["gpu_ms"])
             inv.append(c["info"]["selinv_ms"])
+            if args.points:
+                t = time.perf_counter()
+                cp = ds.covariance(with_points=True)
+                pwall.append(1e3 * (time.perf_counter() - t))
+                pdev.append(cp["info"]["gpu_ms"])
+                pts.append(cp["info"]["points_ms"])
         info = c["info"]
         ds.close()
         r = {"workload": name, "scene": note, "gpu": gpu_state(), "N": s["num_observations"],
@@ -71,6 +104,14 @@ def main():
              "covariance_gpu_ms": spread(dev), "selinv_gpu_ms": spread(inv),
              "covariance_over_lm_round": round(statistics.median(dev) / round_ms, 3),
              "sigma2": info["sigma2"], "std_camera": [float(x) for x in c["std_camera"]]}
+        if args.points:
+            n_pts = int(sc.problem.n_points)
+            r.update({"P": n_pts, "points_copy_mb": round(72 * n_pts / 1e6, 3),
+                      "covariance_points_wall_ms": spread(pwall), "covariance_points_gpu_ms": spread(pdev),
+                      "points_gpu_ms": spread(pts), "points_d2h_copy_ms": spread(d2h_copy_ms(9 * n_pts, args.reps)),
+                      "points_over_lm_round": round(statistics.median(pts) / round_ms, 3),
+                      "median_std_points": [float(x) for x in np.median(cp["std_points"][np.any(cp["points"] != 0,
+                                                                                                 axis=(1, 2))], axis=0)]})
         print(json.dumps(r))
         sys.stdout.flush()
         results.append(r)
