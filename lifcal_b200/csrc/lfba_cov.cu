@@ -150,6 +150,9 @@ __global__ void k_cov_gather(Dev d, const double* __restrict__ Z, double* __rest
 template <int NC>
 __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restrict__ Z, double* __restrict__ out) {
   const SkyMap sky{d.band, d.np6};
+  const int cur = d.st->cur;
+  const double* __restrict__ recs = d.rec[cur];
+  const double* __restrict__ frames = d.frames[cur];
   for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < d.P; p += gridDim.x * blockDim.x) {
     double Sg[6] = {0, 0, 0, 0, 0, 0};  // lower triangle: 00 10 11 20 21 22
     const int cp = d.refine_points && d.st->solve_ok && d.pt_active[p] ? d.pt_coupled[p] : -2;
@@ -165,6 +168,14 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
       double Q[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
       if (d.refine_poses) {
         const int t0 = d.pt_trk_begin[p], t1 = d.pt_trk_begin[p + 1];
+        // V of track t (frame f), recomputed as the assembly computed it (track_v)
+        const double* X = d.points[cur] + 3 * (size_t)p;
+        const double Xp[3] = {X[0], X[1], X[2]};
+        auto track_V = [&](int t, int f, double V[18]) {
+          double A[6], m[9];
+          load_record<6, false>(recs + (size_t)t * rec_stride(NC), A);
+          track_v(A, frames + (size_t)f * kFrameStride, Xp, m, V);
+        };
         for (int a = t0; a < t1; ++a) {
           const int fa = d.trk_frame[a];
           if (fa == d.gauge_frame) continue;
@@ -194,12 +205,7 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
             const int fb = d.trk_frame[b];
             if (fb >= fa || fb == d.gauge_frame) continue;
             double Vb[18];
-            const double* Vp = d.vw + (size_t)b * kVWStride;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) ldg256(Vp + 4 * k, Vb + 4 * k);
-            const double2 v2 = __ldg(reinterpret_cast<const double2*>(Vp) + 8);
-            Vb[16] = v2.x;
-            Vb[17] = v2.y;
+            track_V(b, fb, Vb);
 #pragma unroll
             for (int i = 0; i < 6; ++i) {
               const double* zr = Z + zrow(i) + 6 * fb;
@@ -212,14 +218,7 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
             }
           }
           double Va[18];
-          {
-            const double* Vp = d.vw + (size_t)a * kVWStride;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) ldg256(Vp + 4 * k, Va + 4 * k);
-            const double2 v2 = __ldg(reinterpret_cast<const double2*>(Vp) + 8);
-            Va[16] = v2.x;
-            Va[17] = v2.y;
-          }
+          track_V(a, fa, Va);
 #pragma unroll
           for (int k = 0; k < 18; ++k) y[k] *= 2.0;
           // diagonal block Z[fa, fa], read from its lower triangle
@@ -242,7 +241,7 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
             }
         }
       }
-      // camera-camera (the outer loop unrolled as well gives 255 registers and spills; rolled: 128, none)
+      // camera-camera (the outer loop unrolled as well gives 255 registers and spills; rolled: at most 166, none)
 #pragma unroll 1
       for (int c1 = 0; c1 < NC; ++c1) {
         const int r1 = d.cam_red[c1];

@@ -10,7 +10,6 @@
 //   rec      double[2][T*REC] per-track normal-equation blocks in the camera frame (A 6, b 3, C 3xNC),
 //                          double-buffered: accepted state / candidate
 //   pdata    double[P*40] per-point Schur data (inverse of the damped 3x3, gradient, damping, camera coupling)
-//   vw       double[T*36] per-track pose-point coupling V (6x3) and V*Hpp^-1 (6x3)
 //   S        skyline lower-triangular reduced system [poses 6F | coupled points 3Pc | camera | rhs row]
 // Parameters are double-buffered (accepted x / candidate x+) so that accept/reject is an index flip on device.
 #pragma once
@@ -54,7 +53,6 @@ __device__ __forceinline__ void load_record(const double* __restrict__ p, double
 #endif
 
 constexpr int kPointStride = 40;  // pdata: Hinv(6) gp(3) dmp(3) Hcp(3*NC<=27) pad
-constexpr int kVWStride = 36;     // vw: V(18: 6x3 row-major) W(18)
 constexpr int kMaxLog = 1024;
 constexpr int kTile = 64;         // Cholesky tile
 
@@ -204,7 +202,6 @@ struct Dev {
   double* camsum[2];   // [64]: Hcc (lower, NC*(NC+1)/2), gc (NC), cost
   double* pdata;
   double* pscale;      // [3P] Jacobi scale of the point columns
-  double* vw;
   double* frame_part;  // [F * frame_splits * (39 + 6 NC)] partial sums of k_frame_all when frames are split over CTAs
   // reduced system
   double* S;           // skyline storage

@@ -791,8 +791,12 @@ __global__ void __launch_bounds__(128) k_frame_all(Dev d) {
     for (int k = 0; k < 3; ++k) ldg256(d.pdata + (size_t)p * kPointStride + 4 * k, pd + 4 * k);  // 320-byte records
     const double A[6] = {rc[0], rc[1], rc[2], rc[3], rc[4], rc[5]};
     const double b[3] = {rc[6], rc[7], rc[8]};
-    double m[9];
-    track_M(fe, points + 3 * (size_t)p, m);
+    double m[9], V[18], W[18];
+    track_v(A, fe, points + 3 * (size_t)p, m, V);
+    {
+      const double Hi[6] = {pd[0], pd[1], pd[2], pd[3], pd[4], pd[5]};
+      track_w(Hi, V, W);
+    }
     double AM[18];
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
@@ -806,33 +810,6 @@ __global__ void __launch_bounds__(128) k_frame_all(Dev d) {
     AM[1 * 6 + 3] = A[1]; AM[1 * 6 + 4] = A[3]; AM[1 * 6 + 5] = A[4];
     AM[2 * 6 + 3] = A[2]; AM[2 * 6 + 4] = A[4]; AM[2 * 6 + 5] = A[5];
     auto Mt = [&](int a, int i) -> double { return a < 3 ? m[3 * a + i] : (a - 3 == i ? 1.0 : 0.0); };
-    const double* R = fe;
-    double AR[9];
-#pragma unroll
-    for (int j = 0; j < 3; ++j) {
-      AR[0 + j] = A[0] * R[j] + A[1] * R[3 + j] + A[2] * R[6 + j];
-      AR[3 + j] = A[1] * R[j] + A[3] * R[3 + j] + A[4] * R[6 + j];
-      AR[6 + j] = A[2] * R[j] + A[4] * R[3 + j] + A[5] * R[6 + j];
-    }
-    double V[18], W[18];
-    const double Hi[6] = {pd[0], pd[1], pd[2], pd[3], pd[4], pd[5]};
-#pragma unroll
-    for (int a = 0; a < 6; ++a) {
-#pragma unroll
-      for (int j = 0; j < 3; ++j) V[3 * a + j] = Mt(a, 0) * AR[j] + Mt(a, 1) * AR[3 + j] + Mt(a, 2) * AR[6 + j];
-      sym3_vec(Hi, V + 3 * a, W + 3 * a);
-    }
-    {  // V | W: 288 bytes, 32-byte aligned
-      double* vwp = d.vw + (size_t)t * kVWStride;
-      double vwv[36];
-#pragma unroll
-      for (int k = 0; k < 18; ++k) {
-        vwv[k] = V[k];
-        vwv[18 + k] = W[k];
-      }
-#pragma unroll
-      for (int k = 0; k < 9; ++k) stg256(vwp + 4 * k, vwv[4 * k], vwv[4 * k + 1], vwv[4 * k + 2], vwv[4 * k + 3]);
-    }
     const double gp[3] = {pd[6], pd[7], pd[8]};
     {
       int h = 0;
@@ -910,41 +887,47 @@ __global__ void __launch_bounds__(128) k_frame_finish(Dev d, int nsplit) {
   frame_all_scatter<NC>(d, f, v, sv);
 }
 
-// Per co-visible frame pair (f1 > f2), one warp: S[f1, f2] = -sum_p W_{p,f1} V_{p,f2}^T.
+// Per co-visible frame pair (f1 > f2): S[f1, f2] = -sum_p W_{p,f1} V_{p,f2}^T. V and W of both tracks are recomputed
+// from the track records, the two frame-table entries and the point (track_v / track_w: the bits k_frame_all uses).
+template <int NC>
 __global__ void __launch_bounds__(256) k_pairs(Dev d) {
   LmState* st = d.st;
   if (linear_phase_idle(st)) return;
+  const int cur = st->cur;
   // one CTA per pair, 1..8 warps (the launcher picks the width so that a rank with few pairs still fills the machine)
   const int pair = blockIdx.x, lane = threadIdx.x & 31, wrp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  const int f1 = d.pair_f1[pair], f2 = d.pair_f2[pair];
   __shared__ double sred[8][36];
+  __shared__ double fe[2][kFrameStride];
+  for (int k = threadIdx.x; k < 2 * kFrameStride; k += blockDim.x)  // the CTA may be a single warp
+    fe[k / kFrameStride][k % kFrameStride] = d.frames[cur][(size_t)(k < kFrameStride ? f1 : f2) * kFrameStride + k % kFrameStride];
+  __syncthreads();
+  const double* __restrict__ recs = d.rec[cur];
+  const double* __restrict__ points = d.points[cur];
   double acc[36];
 #pragma unroll
   for (int v = 0; v < 36; ++v) acc[v] = 0.0;
   for (int i = d.pair_begin[pair] + threadIdx.x; i < d.pair_begin[pair + 1]; i += blockDim.x) {
-    // V = first 144 bytes of a 288-byte record (32-byte aligned), W = the second half (16 mod 32): 256-bit loads where
-    // the alignment allows, one 128-bit load at the odd end
-    const double* Vp = d.vw + (size_t)d.pair_t2[i] * kVWStride;
-    const double* Wp = d.vw + (size_t)d.pair_t1[i] * kVWStride + 18;
-    double w[18], v[18];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) ldg256(Vp + 4 * k, v + 4 * k);
+    const int t1 = d.pair_t1[i], t2 = d.pair_t2[i];
+    const int p = d.trk_point[t1];
+    const double* X = points + 3 * (size_t)p;
+    double w[18], v[18], m[9];
     {
-      const double2 t2 = __ldg(reinterpret_cast<const double2*>(Vp + 16));
-      v[16] = t2.x;
-      v[17] = t2.y;
-      const double2 t3 = __ldg(reinterpret_cast<const double2*>(Wp));
-      w[0] = t3.x;
-      w[1] = t3.y;
+      double A[6], Hi[6];
+      load_record<6, false>(recs + (size_t)t1 * rec_stride(NC), A);
+      track_v(A, fe[0], X, m, v);
+      const double* pd = d.pdata + (size_t)p * kPointStride;  // Hpp^-1 leads the point record
+      load_record<6, false>(pd, Hi);
+      track_w(Hi, v, w);
+      load_record<6, false>(recs + (size_t)t2 * rec_stride(NC), A);
+      track_v(A, fe[1], X, m, v);
     }
-#pragma unroll
-    for (int k = 0; k < 4; ++k) ldg256(Wp + 2 + 4 * k, w + 2 + 4 * k);
 #pragma unroll
     for (int a = 0; a < 6; ++a)
 #pragma unroll
       for (int b = 0; b < 6; ++b)
         acc[6 * a + b] += w[3 * a] * v[3 * b] + w[3 * a + 1] * v[3 * b + 1] + w[3 * a + 2] * v[3 * b + 2];
   }
-  const int f1 = d.pair_f1[pair], f2 = d.pair_f2[pair];
 #pragma unroll
   for (int v = 0; v < 36; ++v) {
     const double s = warp_sum(acc[v]);
@@ -1249,18 +1232,16 @@ __global__ void __launch_bounds__(128) k_point_step(Dev d) {
       h[1] += pd[13 + 3 * c] * yc;
       h[2] += pd[14 + 3 * c] * yc;
     }
-    if (d.refine_poses) {
+    if (d.refine_poses) {  // sum_t V_t^T y_f, V_t recomputed from the track's A block, its frame entry and X
+      const double* __restrict__ frames = d.frames[cur];
+      const double* X = d.points[cur] + 3 * (size_t)p;
+      const double Xp[3] = {X[0], X[1], X[2]};
       for (int t = d.pt_trk_begin[p]; t < d.pt_trk_begin[p + 1]; ++t) {
-        double V[18];
-        {  // 144 bytes at a 32-byte aligned address: four 256-bit loads + one 128-bit
-          const double* Vp = d.vw + (size_t)t * kVWStride;
-#pragma unroll
-          for (int k = 0; k < 4; ++k) ldg256(Vp + 4 * k, V + 4 * k);
-          const double2 v2 = __ldg(reinterpret_cast<const double2*>(Vp) + 8);
-          V[16] = v2.x;
-          V[17] = v2.y;
-        }
-        const double* yf = y + 6 * d.trk_frame[t];
+        const int f = d.trk_frame[t];
+        double V[18], m[9], A[6];
+        load_record<6, false>(d.rec[cur] + (size_t)t * rec_stride(NC), A);
+        track_v(A, frames + (size_t)f * kFrameStride, Xp, m, V);
+        const double* yf = y + 6 * f;
 #pragma unroll
         for (int a = 0; a < 6; ++a) {
           h[0] += V[3 * a] * yf[a];
@@ -1458,7 +1439,7 @@ int launch_assembly(const Dev& d, int frame_splits, cudaStream_t s) {
     if (d.refine_points && d.npairs > 0) {
       int wpp = 1;  // warps per pair: enough CTAs x warps to cover the SMs a few times
       while (wpp < 8 && (long long)d.npairs * wpp < 4096) wpp *= 2;
-      k_pairs<<<d.npairs, 32 * wpp, 0, s>>>(d);
+      LFBA_DISPATCH_NC(d.NC, (k_pairs<NC><<<d.npairs, 32 * wpp, 0, s>>>(d)));
       ++launches;
     }
   }

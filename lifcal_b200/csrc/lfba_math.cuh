@@ -614,6 +614,47 @@ LFBA_HD void sym3_vec(const double a[6], const double x[3], double y[3]) {
   y[2] = a[2] * x[0] + a[4] * x[1] + a[5] * x[2];
 }
 
+// a0 b0 + a1 b1 + a2 b2 with the roundings nvcc --fmad=true gives that expression (the middle product rounded, the
+// other two fused), written out so that every kernel inlining the helpers below computes the same bits
+LFBA_HD double dot3_fma(double a0, double b0, double a1, double b1, double a2, double b2) {
+  return fma(a2, b2, fma(a0, b0, a1 * b1));
+}
+
+// Pose-point coupling of one track, V = M^T A R (6 x 3, row-major: the pose x point block of J^T W J), recomputed
+// where it is used instead of being stored per track. A is the track's 3 x 3 block (upper: 00 01 02 11 12 22), fe its
+// frame-table entry (R, dR/da0..2), X the point. Also gives m, the 3 x 3 part of M = [dR0 X, dR1 X, dR2 X, I3]
+// (m[3 a + i] = (dR_a X)_i). Rows 3..5 are A R itself.
+LFBA_HD void track_v(const double A[6], const double* fe, const double* X, double m[9], double V[18]) {
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    const double* dR = fe + 9 * (a + 1);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) m[3 * a + i] = dot3_fma(dR[3 * i], X[0], dR[3 * i + 1], X[1], dR[3 * i + 2], X[2]);
+  }
+  const double* R = fe;
+#pragma unroll
+  for (int j = 0; j < 3; ++j) {
+    V[9 + j] = dot3_fma(A[0], R[j], A[1], R[3 + j], A[2], R[6 + j]);
+    V[12 + j] = dot3_fma(A[1], R[j], A[3], R[3 + j], A[4], R[6 + j]);
+    V[15 + j] = dot3_fma(A[2], R[j], A[4], R[3 + j], A[5], R[6 + j]);
+  }
+#pragma unroll
+  for (int a = 0; a < 3; ++a)
+#pragma unroll
+    for (int j = 0; j < 3; ++j)
+      V[3 * a + j] = dot3_fma(m[3 * a], V[9 + j], m[3 * a + 1], V[12 + j], m[3 * a + 2], V[15 + j]);
+}
+// W = V Hpp^-1 (6 x 3) from V and the inverse of the point's damped 3 x 3 block (upper triangle)
+LFBA_HD void track_w(const double Hi[6], const double V[18], double W[18]) {
+#pragma unroll
+  for (int a = 0; a < 6; ++a) {
+    const double* v = V + 3 * a;
+    W[3 * a] = dot3_fma(Hi[0], v[0], Hi[1], v[1], Hi[2], v[2]);
+    W[3 * a + 1] = dot3_fma(Hi[1], v[0], Hi[3], v[1], Hi[4], v[2]);
+    W[3 * a + 2] = dot3_fma(Hi[2], v[0], Hi[4], v[1], Hi[5], v[2]);
+  }
+}
+
 // distance constraint (src/BundleAdjustment/BundleAdjustment.h:262-267): r = (|p1 - p2| - d) / (sigma + 1e-6),
 // j = d r / d p1 = -(d r / d p2)
 LFBA_HD void distance_eval(const double* p1, const double* p2, double dist, double sigma, double& r, double j[3]) {

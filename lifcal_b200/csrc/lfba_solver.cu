@@ -146,7 +146,7 @@ struct Solver {
   DevBuf<int64_t> row_off;
   DevBuf<double> c_dist, c_sigma;
   DevBuf<double> camera0, views0, points0;  // parameters given by the caller: every run() starts from them
-  DevBuf<double> camera[2], views[2], points[2], lens, frames[2], rec[2], camsum[2], pdata, pscale, vw, pstep;
+  DevBuf<double> camera[2], views[2], points[2], lens, frames[2], rec[2], camsum[2], pdata, pscale, pstep;
   DevBuf<double> redbuf;  // S | g | gfull | hdiag | sys_scalars   (one all-reduce)
   DevBuf<double> rscale, rdamp, y, eval_scalars, part_eval, part_pts, part_step, part_ls, frame_part;
   DevBuf<CamModel> cm_buf;
@@ -354,7 +354,6 @@ struct Solver {
     pdata.alloc((size_t)P * kPointStride);
     pdata.zero(stream);
     pscale.alloc((size_t)3 * P);
-    vw.alloc((size_t)std::max(1, T) * kVWStride);
     if (recalib) {
       pstep.alloc((size_t)3 * P);
       pstep.zero(stream);
@@ -435,7 +434,7 @@ struct Solver {
       d.frames[b] = frames[b].p; d.rec[b] = rec[b].p; d.camsum[b] = camsum[b].p;
     }
     d.lens = lens.p; d.lens_xy = ix.lens_xy.p; d.cm_buf = cm_buf.p;
-    d.pdata = pdata.p; d.pscale = pscale.p; d.vw = vw.p; d.pstep = pstep.p;
+    d.pdata = pdata.p; d.pscale = pscale.p; d.pstep = pstep.p;
     d.S = redbuf.p; d.row_off = row_off.p; d.row_c0 = row_c0.p;
     d.g = redbuf.p + S_len; d.gfull = d.g + n; d.hdiag = d.gfull + n; d.sys_scalars = d.hdiag + n;
     d.rscale = rscale.p; d.rdamp = rdamp.p; d.y = y.p; d.eval_scalars = eval_scalars.p;
