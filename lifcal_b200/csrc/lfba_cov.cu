@@ -138,14 +138,16 @@ __global__ void k_cov_gather(Dev d, const double* __restrict__ Z, double* __rest
 
 // Per-point 3 x 3 blocks. An eliminated point p (pdata written by the undamped k_points) has, with Hi = Hpp^-1 and u the
 // point's n x 3 coupling column of J^T W J (V_t^T of its tracks in pose rows, Hcp in camera rows),
-//     Sigma_pp = Hi + Hi Q Hi,   Q = u^T Z u = sum_{a,b} V_a^T Z[f_a, f_b] V_b + (M + M^T) + Hcp^T Z[cam, cam] Hcp,
-//     M = sum_a V_a^T Z[f_a, cam] Hcp
-// (block inverse of [[S, u], [u^T, Hpp]]). Q is symmetric, so it is its own symmetric part sym(X) = (X + X^T) / 2, and
-// sym(V_a^T Z_ab V_b) = sym(V_b^T Z_ba V_a): with one track per (point, frame),
-//     Q = sym( sum_a V_a^T y_a ) + Hcp^T Z[cam, cam] Hcp,   y_a = Z[f_a, f_a] V_a + 2 (sum_{f_b < f_a} Z[f_a, f_b] V_b + Z[f_a, cam] Hcp)
-// reads only lower blocks of Z (row f_a, columns 6 f_b .. contiguous) and does half the pairs, 108 FMA each. Tracks in
-// the gauge frame are skipped: that pose is not a parameter, and Z holds identity on its rows. Frames of one point are at
-// most `band` apart, so every Z[f_a, f_b] lies in the envelope. A coupled point's block is its diagonal block of Z. One
+//     Sigma_pp = Hi + Hi Q Hi,   Q = u^T Z u
+// (block inverse of [[S, u], [u^T, Hpp]]). With w = u Hi (W_t = V_t Hi = M_t^T (B_t Hi) in pose rows, T_p^T = Hcp Hi in
+// camera rows: the point record holds T_p), Hi Q Hi = w^T Z w =: Q~, and
+//     Q~ = sum_{a,b} W_a^T Z[f_a, f_b] W_b + (N + N^T) + T_p Z[cam, cam] T_p^T,   N = sum_a W_a^T Z[f_a, cam] T_p^T.
+// Q~ is symmetric, so it is its own symmetric part sym(X) = (X + X^T) / 2, and sym(W_a^T Z_ab W_b) = sym(W_b^T Z_ba W_a):
+// with one track per (point, frame),
+//     Q~ = sym( sum_a W_a^T y_a ) + T_p Z[cam, cam] T_p^T,   y_a = Z[f_a, f_a] W_a + 2 (sum_{f_b < f_a} Z[f_a, f_b] W_b + Z[f_a, cam] T_p^T)
+// and Sigma_pp = Hi + sym(Q~). This reads only lower blocks of Z (row f_a, columns 6 f_b .. contiguous) and does half the
+// pairs, 108 FMA each. Tracks in the gauge frame are skipped: that pose is not a parameter, and Z holds identity on its
+// rows. Frames of one point are at most `band` apart, so every Z[f_a, f_b] lies in the envelope. A coupled point's block is its diagonal block of Z. One
 // thread per point.
 template <int NC>
 __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restrict__ Z, double* __restrict__ out) {
@@ -164,17 +166,22 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
         for (int j = 0; j <= i; ++j, ++h) Sg[h] = Z[sky_off(sky, r0 + i, r0 + j)];
     } else if (cp == -1) {
       const double* __restrict__ pd = d.pdata + (size_t)p * kPointStride;
-      const double* __restrict__ Hc = pd + 12;  // Hcp[3 c + j]; columns with cam_red[c] < 0 are skipped
+      const double* __restrict__ Tp = pd + 12;  // T_p[j][c] at 3 c + j; columns with cam_red[c] < 0 are skipped
       double Q[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
       if (d.refine_poses) {
         const int t0 = d.pt_trk_begin[p], t1 = d.pt_trk_begin[p + 1];
-        // V of track t (frame f), recomputed as the assembly computed it (track_v)
+        // W of track t (frame f) = M^T (B Hi), from the helpers the assembly uses
         const double* X = d.points[cur] + 3 * (size_t)p;
         const double Xp[3] = {X[0], X[1], X[2]};
-        auto track_V = [&](int t, int f, double V[18]) {
-          double A[6], m[9];
+        auto track_W = [&](int t, int f, double W[18]) {
+          double A[6], m[9], B[9], K[9], Hi[6];
+          const double* fe = frames + (size_t)f * kFrameStride;
           load_record<6, false>(recs + (size_t)t * rec_stride(NC), A);
-          track_v(A, frames + (size_t)f * kFrameStride, Xp, m, V);
+          track_m(fe, Xp, m);
+          track_b(A, fe, B);
+          load_record<6, false>(pd, Hi);
+          mat3_sym3(B, Hi, K);
+          mt_mat(m, K, W);
         };
         for (int a = t0; a < t1; ++a) {
           const int fa = d.trk_frame[a];
@@ -191,7 +198,7 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
             const int r = d.cam_red[c];
             if (r < 0) continue;
             const double* zr = Z + sky.border_row(r - d.np6) + 6 * fa;
-            const double h0 = Hc[3 * c], h1 = Hc[3 * c + 1], h2 = Hc[3 * c + 2];
+            const double h0 = Tp[3 * c], h1 = Tp[3 * c + 1], h2 = Tp[3 * c + 2];
 #pragma unroll
             for (int i = 0; i < 6; ++i) {
               const double z = zr[i];
@@ -204,8 +211,8 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
           for (int b = t0; b < t1; ++b) {
             const int fb = d.trk_frame[b];
             if (fb >= fa || fb == d.gauge_frame) continue;
-            double Vb[18];
-            track_V(b, fb, Vb);
+            double Wb[18];
+            track_W(b, fb, Wb);
 #pragma unroll
             for (int i = 0; i < 6; ++i) {
               const double* zr = Z + zrow(i) + 6 * fb;
@@ -213,12 +220,12 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
               for (int j = 0; j < 6; ++j) {
                 const double z = zr[j];
 #pragma unroll
-                for (int k = 0; k < 3; ++k) y[3 * i + k] += z * Vb[3 * j + k];
+                for (int k = 0; k < 3; ++k) y[3 * i + k] += z * Wb[3 * j + k];
               }
             }
           }
-          double Va[18];
-          track_V(a, fa, Va);
+          double Wa[18];
+          track_W(a, fa, Wa);
 #pragma unroll
           for (int k = 0; k < 18; ++k) y[k] *= 2.0;
           // diagonal block Z[fa, fa], read from its lower triangle
@@ -228,7 +235,7 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
             for (int j = 0; j < 6; ++j) {
               const double z = i >= j ? Z[zrow(i) + 6 * fa + j] : Z[zrow(j) + 6 * fa + i];
 #pragma unroll
-              for (int k = 0; k < 3; ++k) y[3 * i + k] += z * Va[3 * j + k];
+              for (int k = 0; k < 3; ++k) y[3 * i + k] += z * Wa[3 * j + k];
             }
 #pragma unroll
           for (int i = 0; i < 3; ++i)
@@ -236,7 +243,7 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
             for (int j = 0; j < 3; ++j) {
               double m = 0.0;
 #pragma unroll
-              for (int k = 0; k < 6; ++k) m += Va[3 * k + i] * y[3 * k + j];
+              for (int k = 0; k < 6; ++k) m += Wa[3 * k + i] * y[3 * k + j];
               Q[3 * i + j] += m;
             }
         }
@@ -253,34 +260,19 @@ __global__ void __launch_bounds__(128) k_cov_points(Dev d, const double* __restr
           if (r2 < 0) continue;
           const double z = sym_at(Z, sky, r1, r2);
 #pragma unroll
-          for (int j = 0; j < 3; ++j) y[j] += z * Hc[3 * c2 + j];
+          for (int j = 0; j < 3; ++j) y[j] += z * Tp[3 * c2 + j];
         }
 #pragma unroll
         for (int i = 0; i < 3; ++i)
 #pragma unroll
-          for (int j = 0; j < 3; ++j) Q[3 * i + j] += Hc[3 * c1 + i] * y[j];
+          for (int j = 0; j < 3; ++j) Q[3 * i + j] += Tp[3 * c1 + i] * y[j];
       }
-      // Sigma = Hi + Hi sym(Q) Hi
-      const double Hi[9] = {pd[0], pd[1], pd[2], pd[1], pd[3], pd[4], pd[2], pd[4], pd[5]};
-      double T[9];
-#pragma unroll
-      for (int i = 0; i < 3; ++i)
-#pragma unroll
-        for (int j = 0; j < 3; ++j) {
-          double v = 0.0;
-#pragma unroll
-          for (int k = 0; k < 3; ++k) v += Hi[3 * i + k] * (0.5 * (Q[3 * k + j] + Q[3 * j + k]));
-          T[3 * i + j] = v;
-        }
+      // Sigma = Hi + sym(Q~)
+      const double Hi[6] = {pd[0], pd[1], pd[2], pd[3], pd[4], pd[5]};
 #pragma unroll
       for (int i = 0, h = 0; i < 3; ++i)
 #pragma unroll
-        for (int j = 0; j <= i; ++j, ++h) {
-          double v = Hi[3 * i + j];
-#pragma unroll
-          for (int k = 0; k < 3; ++k) v += T[3 * i + k] * Hi[3 * k + j];
-          Sg[h] = v;
-        }
+        for (int j = 0; j <= i; ++j, ++h) Sg[h] = Hi[j * 3 - j * (j + 1) / 2 + i] + 0.5 * (Q[3 * i + j] + Q[3 * j + i]);
     }
     double* o = out + 9 * (size_t)p;
     o[0] = Sg[0]; o[1] = Sg[1]; o[2] = Sg[3];

@@ -9,7 +9,7 @@
 //   trk_*    int32[T]     point, frame, first observation of each track (+ begin[T])
 //   rec      double[2][T*REC] per-track normal-equation blocks in the camera frame (A 6, b 3, C 3xNC),
 //                          double-buffered: accepted state / candidate
-//   pdata    double[P*40] per-point Schur data (inverse of the damped 3x3, gradient, damping, camera coupling)
+//   pdata    double[P*40] per-point Schur data (inverse of the damped 3x3, gradient, damping, inverse x camera coupling)
 //   S        skyline lower-triangular reduced system [poses 6F | coupled points 3Pc | camera | rhs row]
 // Parameters are double-buffered (accepted x / candidate x+) so that accept/reject is an index flip on device.
 #pragma once
@@ -52,7 +52,7 @@ __device__ __forceinline__ void load_record(const double* __restrict__ p, double
 }
 #endif
 
-constexpr int kPointStride = 40;  // pdata: Hinv(6) gp(3) dmp(3) Hcp(3*NC<=27) pad
+constexpr int kPointStride = 40;  // pdata: Hinv(6) gp(3) dmp(3) T_p = Hinv Hcp^T (3*NC<=27, [3 c + j]) pad
 constexpr int kMaxLog = 1024;
 constexpr int kTile = 64;         // Cholesky tile
 

@@ -11,10 +11,10 @@
 //                          block (Hcc, gc) + cost.  The Jacobian never leaves registers.
 //      k_reduce_eval       deterministic reduction of the per-CTA partials; candidate scalars
 //   C1 k_control_accept    step tests, rho, accept/reject (buffer flip), radius update   [device-resident LM]
-//   B  k_points            per point: Hpp, g_p, Hcp; damping; 3x3 inverse; camera-camera Schur term
-//      k_frame_all         per frame: pose diagonal block, pose gradient, camera-pose block (Schur-corrected), V and
-//                          W = V Hpp^-1 (+ k_frame_finish when a frame's tracks are split over several CTAs)
-//      k_pairs             per co-visible frame pair: -sum_p W_{p,f1} V_{p,f2}^T
+//   B  k_points            per point: Hpp, g_p, Hcp; damping; 3x3 inverse; T_p = Hpp^-1 Hcp^T; camera-camera Schur term
+//      k_frame_all         per frame: pose diagonal block, pose gradient, camera-pose block, Schur-corrected in the
+//                          camera frame (+ k_frame_finish when a frame's tracks are split over several CTAs)
+//      k_pairs             per co-visible frame pair: -sum_p M1^T (B1 Hpp^-1 B2^T) M2
 //      k_coupled, k_constraints, k_add_camera
 //   C2 k_finalize          Jacobi scaling (iteration 0), gradient norms, iteration row, termination tests,
 //                          LM damping of the reduced system
@@ -596,7 +596,7 @@ __global__ void __launch_bounds__(256) k_ls_apply_reduced(Dev d) {
 // B. system assembly at the accepted state
 // ================================================================================================
 // Per point: Hpp = sum_t R^T A_t R, g_p = sum_t R^T b_t, Hcp = sum_t C_t^T R  (E-block of SchurEliminator),
-// Jacobi scale (iteration 0), LM damping, inverse of the damped block, camera-camera Schur term.
+// Jacobi scale (iteration 0), LM damping, inverse Hi of the damped block, T_p = Hi Hcp^T, camera-camera Schur term.
 template <int NC>
 __global__ void __launch_bounds__(128) k_points(Dev d) {
   LmState* st = d.st;
@@ -669,24 +669,11 @@ __global__ void __launch_bounds__(128) k_points(Dev d) {
       acc[NH + NC + 1] += 1.0;
       for (int k = 0; k < 6; ++k) Hi[k] = 0.0;
     }
-    {  // 320-byte record, 32-byte aligned: ten 256-bit stores (forty 8-byte stores cost forty times 32 L1 wavefronts per warp)
-      double pv[kPointStride];
-#pragma unroll
-      for (int k = 0; k < 6; ++k) pv[k] = Hi[k];
-#pragma unroll
-      for (int k = 0; k < 3; ++k) {
-        pv[6 + k] = gp[k];
-        pv[9 + k] = dmp[k];
-      }
-#pragma unroll
-      for (int k = 0; k < kPointStride - 12; ++k) pv[12 + k] = k < 3 * NC ? Hcp[k] : 0.0;
-#pragma unroll
-      for (int k = 0; k < kPointStride / 4; ++k) stg256(pd + 4 * k, pv[4 * k], pv[4 * k + 1], pv[4 * k + 2], pv[4 * k + 3]);
-    }
-    // camera-camera Schur term: -(Hcp Hi) Hcp^T, -(Hcp Hi) g_p
+    // T_p = Hi Hcp^T (NC x 3 here: Tm[3 c + j]): the point record's camera coupling and the camera-camera Schur term
     double Tm[3 * NC];
 #pragma unroll
     for (int c = 0; c < NC; ++c) sym3_vec(Hi, Hcp + 3 * c, Tm + 3 * c);
+    // camera-camera Schur term: -(Hcp Hi) Hcp^T, -(Hcp Hi) g_p
     int h = 0;
 #pragma unroll
     for (int c1 = 0; c1 < NC; ++c1)
@@ -698,6 +685,20 @@ __global__ void __launch_bounds__(128) k_points(Dev d) {
 #pragma unroll
     for (int c = 0; c < NC; ++c) acc[NH + c] -= Tm[3 * c] * gp[0] + Tm[3 * c + 1] * gp[1] + Tm[3 * c + 2] * gp[2];
     acc[NH + NC] += gp[0] * gp[0] + gp[1] * gp[1] + gp[2] * gp[2];
+    {  // 320-byte record, 32-byte aligned: ten 256-bit stores (forty 8-byte stores cost forty times 32 L1 wavefronts per warp)
+      double pv[kPointStride];
+#pragma unroll
+      for (int k = 0; k < 6; ++k) pv[k] = Hi[k];
+#pragma unroll
+      for (int k = 0; k < 3; ++k) {
+        pv[6 + k] = gp[k];
+        pv[9 + k] = dmp[k];
+      }
+#pragma unroll
+      for (int k = 0; k < kPointStride - 12; ++k) pv[12 + k] = k < 3 * NC ? Tm[k] : 0.0;
+#pragma unroll
+      for (int k = 0; k < kPointStride / 4; ++k) stg256(pd + 4 * k, pv[4 * k], pv[4 * k + 1], pv[4 * k + 2], pv[4 * k + 3]);
+    }
     gmax = fmax(gmax, fmax(fabs(gp[0]), fmax(fabs(gp[1]), fabs(gp[2]))));
   }
   block_reduce_store<NV>(acc, d.part_pts + (size_t)blockIdx.x * 64, red);
@@ -755,6 +756,10 @@ __global__ void __launch_bounds__(128) k_frame_all(Dev d) {
   __shared__ double fe[kFrameStride];
   __shared__ double red[4 * NV];
   __shared__ double out[NV];
+  // The NP pose-side sums (each updated once per track) are kept per thread in shared memory, [v][thread]: the
+  // registers then hold only the 6 NC camera-pose sums, and the loop-carried accumulators no longer spill.
+  __shared__ double sacc[NP * 128];  // launched with 128 threads
+  double* const my = sacc + threadIdx.x;
   for (int f = blockIdx.y; f < d.F; f += gridDim.y) {  // (one frame per CTA unless F exceeds the grid limit)
   __syncthreads();
   if (threadIdx.x < kFrameStride) fe[threadIdx.x] = d.frames[cur][(size_t)f * kFrameStride + threadIdx.x];
@@ -762,6 +767,8 @@ __global__ void __launch_bounds__(128) k_frame_all(Dev d) {
   double acc[NV];
 #pragma unroll
   for (int v = 0; v < NV; ++v) acc[v] = 0.0;
+#pragma unroll
+  for (int v = 0; v < NP; ++v) my[128 * v] = 0.0;
   const double* __restrict__ recs = d.rec[cur];
   const double* __restrict__ points = d.points[cur];
   for (int idx = d.frm_begin[f] + split * blockDim.x + threadIdx.x; idx < d.frm_begin[f + 1];
@@ -769,7 +776,7 @@ __global__ void __launch_bounds__(128) k_frame_all(Dev d) {
     const int t = d.frm_trk[idx];
     const int p = d.trk_point[t];
     // first the 3x3 part of the record and of the point data (A, b | Hpp^-1, g_p); the camera parts are loaded after
-    // the pose block is done, so that they are not live across it (255 registers: 93 accumulators + one track)
+    // the pose block is done, so that they are not live across it
     const double* rcp = recs + (size_t)t * RS;
     const double2* pd2 = reinterpret_cast<const double2*>(d.pdata + (size_t)p * kPointStride);
     double rc[12], pd[12];
@@ -791,46 +798,48 @@ __global__ void __launch_bounds__(128) k_frame_all(Dev d) {
     for (int k = 0; k < 3; ++k) ldg256(d.pdata + (size_t)p * kPointStride + 4 * k, pd + 4 * k);  // 320-byte records
     const double A[6] = {rc[0], rc[1], rc[2], rc[3], rc[4], rc[5]};
     const double b[3] = {rc[6], rc[7], rc[8]};
-    double m[9], V[18], W[18];
-    track_v(A, fe, points + 3 * (size_t)p, m, V);
-    {
-      const double Hi[6] = {pd[0], pd[1], pd[2], pd[3], pd[4], pd[5]};
-      track_w(Hi, V, W);
-    }
-    double AM[18];
+    double m[9], B[9];
+    track_m(fe, points + 3 * (size_t)p, m);
+    track_b(A, fe, B);
+    {  // pose block and gradients, the point eliminated in the camera frame: A~ = A - K B^T, b~ = b - K g_p (K = B Hi)
+      double lp[NP];
 #pragma unroll
-    for (int k = 0; k < 3; ++k) {
-      double y[3];
-      sym3_vec(A, m + 3 * k, y);
-      AM[0 * 6 + k] = y[0];
-      AM[1 * 6 + k] = y[1];
-      AM[2 * 6 + k] = y[2];
-    }
-    AM[0 * 6 + 3] = A[0]; AM[0 * 6 + 4] = A[1]; AM[0 * 6 + 5] = A[2];
-    AM[1 * 6 + 3] = A[1]; AM[1 * 6 + 4] = A[3]; AM[1 * 6 + 5] = A[4];
-    AM[2 * 6 + 3] = A[2]; AM[2 * 6 + 4] = A[4]; AM[2 * 6 + 5] = A[5];
-    auto Mt = [&](int a, int i) -> double { return a < 3 ? m[3 * a + i] : (a - 3 == i ? 1.0 : 0.0); };
-    const double gp[3] = {pd[6], pd[7], pd[8]};
-    {
-      int h = 0;
-#pragma unroll
-      for (int a = 0; a < 6; ++a) {
-        const double gva = Mt(a, 0) * b[0] + Mt(a, 1) * b[1] + Mt(a, 2) * b[2];
-#pragma unroll
-        for (int c = 0; c <= a; ++c) {
-          const double hvv = Mt(a, 0) * AM[0 * 6 + c] + Mt(a, 1) * AM[1 * 6 + c] + Mt(a, 2) * AM[2 * 6 + c];
-          acc[h] += hvv - (W[3 * a] * V[3 * c] + W[3 * a + 1] * V[3 * c + 1] + W[3 * a + 2] * V[3 * c + 2]);
-          if (c == a) acc[33 + a] += hvv;
-          ++h;
-        }
-        acc[21 + a] += gva - (W[3 * a] * gp[0] + W[3 * a + 1] * gp[1] + W[3 * a + 2] * gp[2]);
-        acc[27 + a] += gva;
+      for (int v = 0; v < NP; ++v) lp[v] = 0.0;
+      double K[9];
+      {
+        const double Hi[6] = {pd[0], pd[1], pd[2], pd[3], pd[4], pd[5]};
+        mat3_sym3(B, Hi, K);
       }
+      double At[6];
+      track_atilde(A, B, K, At);
+      mt_sym_m_acc(m, At, lp);
+      double bt[3];
+      {
+        const double gp[3] = {pd[6], pd[7], pd[8]};
+        mat3_vec(K, gp, bt);
+      }
+#pragma unroll
+      for (int i = 0; i < 3; ++i) bt[i] = b[i] - bt[i];
+      mt_vec_acc(m, bt, 1.0, lp + 21);
+      mt_vec_acc(m, b, 1.0, lp + 27);
+      // diag(M^T A M), un-complemented
+#pragma unroll
+      for (int a = 0; a < 3; ++a) {
+        double y[3];
+        sym3_vec(A, m + 3 * a, y);
+        lp[33 + a] = dot3_fma(m[3 * a], y[0], m[3 * a + 1], y[1], m[3 * a + 2], y[2]);
+      }
+      lp[36] = A[0];
+      lp[37] = A[3];
+      lp[38] = A[5];
+#pragma unroll
+      for (int v = 0; v < NP; ++v) my[128 * v] += lp[v];
     }
-    // camera-pose block: C_t^T M_t - Hcp W_t^T, streamed in memory order in 256-bit pieces — no register copy of the two
+    // camera-pose block: (C - B T_p)^T M, streamed in memory order in 256-bit pieces — no register copy of the two
     // 3 x NC blocks (they were 104 registers beside the 93 accumulators, most of the spill traffic). C is 3 x NC row-major
     // at doubles 9 .. of the track record: value (i, c) adds C_ic m[3a + i] to entry (c, a < 3) and itself to entry
-    // (c, 3 + i). Hcp is NC x 3 at doubles 12 .. of the point record: value (c, j) subtracts Hcp_cj W[3a + j] from (c, a).
+    // (c, 3 + i). T_p is NC x 3 at doubles 12 .. of the point record: the three values of camera c give (B T_p)_c, whose
+    // projection M^T (B T_p)_c is subtracted from entries (c, 0..5).
     {
       static_assert(RS % 4 == 0, "records are whole 32-byte sectors");
       auto add_c = [&](int k, double v) {  // k: index into C, compile-time after unrolling
@@ -839,10 +848,12 @@ __global__ void __launch_bounds__(128) k_frame_all(Dev d) {
         for (int a = 0; a < 3; ++a) acc[NP + 6 * c + a] = fma(v, m[3 * a + i], acc[NP + 6 * c + a]);
         acc[NP + 6 * c + 3 + i] += v;
       };
-      auto sub_h = [&](int k, double v) {  // k: index into Hcp
+      double bt[3];
+      auto sub_t = [&](int k, double v) {  // k: index into T_p
         const int c = k / 3, jj = k - 3 * c;
 #pragma unroll
-        for (int a = 0; a < 6; ++a) acc[NP + 6 * c + a] = fma(-v, W[3 * a + jj], acc[NP + 6 * c + a]);
+        for (int i = 0; i < 3; ++i) bt[i] = jj == 0 ? B[3 * i] * v : fma(B[3 * i + jj], v, bt[i]);
+        if (jj == 2) mt_vec_acc(m, bt, -1.0, acc + NP + 6 * c);
       };
       add_c(0, rc[9]);
       add_c(1, rc[10]);
@@ -861,10 +872,12 @@ __global__ void __launch_bounds__(128) k_frame_all(Dev d) {
         ldg256(d.pdata + (size_t)p * kPointStride + 4 * q, t4);
 #pragma unroll
         for (int e = 0; e < 4; ++e)
-          if (4 * q + e - 12 < 3 * NC) sub_h(4 * q + e - 12, t4[e]);
+          if (4 * q + e - 12 < 3 * NC) sub_t(4 * q + e - 12, t4[e]);
       }
     }
   }
+#pragma unroll
+  for (int v = 0; v < NP; ++v) acc[v] = my[128 * v];
   block_reduce_store<NV>(acc, out, red);
   if (threadIdx.x < NV) {
     if (nsplit == 1) frame_all_scatter<NC>(d, f, threadIdx.x, out[threadIdx.x]);
@@ -887,8 +900,9 @@ __global__ void __launch_bounds__(128) k_frame_finish(Dev d, int nsplit) {
   frame_all_scatter<NC>(d, f, v, sv);
 }
 
-// Per co-visible frame pair (f1 > f2): S[f1, f2] = -sum_p W_{p,f1} V_{p,f2}^T. V and W of both tracks are recomputed
-// from the track records, the two frame-table entries and the point (track_v / track_w: the bits k_frame_all uses).
+// Per co-visible frame pair (f1 > f2): S[f1, f2] = -sum_p W_{p,f1} V_{p,f2}^T = -sum_p M1^T (B1 Hi B2^T) M2, factored
+// through the 3 x 3 camera-frame product (the helpers k_frame_all uses), from the track records, the two frame-table
+// entries and the point.
 template <int NC>
 __global__ void __launch_bounds__(256) k_pairs(Dev d) {
   LmState* st = d.st;
@@ -911,22 +925,24 @@ __global__ void __launch_bounds__(256) k_pairs(Dev d) {
     const int t1 = d.pair_t1[i], t2 = d.pair_t2[i];
     const int p = d.trk_point[t1];
     const double* X = points + 3 * (size_t)p;
-    double w[18], v[18], m[9];
+    double G[9];
     {
-      double A[6], Hi[6];
+      double A[6], B[9], K[9];
       load_record<6, false>(recs + (size_t)t1 * rec_stride(NC), A);
-      track_v(A, fe[0], X, m, v);
-      const double* pd = d.pdata + (size_t)p * kPointStride;  // Hpp^-1 leads the point record
-      load_record<6, false>(pd, Hi);
-      track_w(Hi, v, w);
+      track_b(A, fe[0], B);
+      {
+        double Hi[6];
+        load_record<6, false>(d.pdata + (size_t)p * kPointStride, Hi);  // Hpp^-1 leads the point record
+        mat3_sym3(B, Hi, K);
+      }
       load_record<6, false>(recs + (size_t)t2 * rec_stride(NC), A);
-      track_v(A, fe[1], X, m, v);
+      track_b(A, fe[1], B);
+      mat3_mat3t(K, B, G);
     }
-#pragma unroll
-    for (int a = 0; a < 6; ++a)
-#pragma unroll
-      for (int b = 0; b < 6; ++b)
-        acc[6 * a + b] += w[3 * a] * v[3 * b] + w[3 * a + 1] * v[3 * b + 1] + w[3 * a + 2] * v[3 * b + 2];
+    double m1[9], m2[9];
+    track_m(fe[0], X, m1);
+    track_m(fe[1], X, m2);
+    mt_mat_m_acc(m1, G, m2, acc);
   }
 #pragma unroll
   for (int v = 0; v < 36; ++v) {
@@ -1208,8 +1224,8 @@ __global__ void __launch_bounds__(1024) k_finalize(Dev d) {
 // ================================================================================================
 // P. steps and candidate
 // ================================================================================================
-// Per point back substitution y_p = Hpp^-1 (g_p - Hpc y_c - sum_t V_t^T y_f), candidate X+ = X - y_p, and the
-// point's share of: model cost change 1/2 y.(g + D y), |step|^2, |x+|^2, g.delta.
+// Per point back substitution y_p = Hpp^-1 (g_p - sum_t V_t^T y_f) - T_p y_c (T_p = Hpp^-1 Hcp^T from k_points),
+// candidate X+ = X - y_p, and the point's share of: model cost change 1/2 y.(g + D y), |step|^2, |x+|^2, g.delta.
 template <int NC>
 __global__ void __launch_bounds__(128) k_point_step(Dev d) {
   LmState* st = d.st;
@@ -1223,37 +1239,35 @@ __global__ void __launch_bounds__(128) k_point_step(Dev d) {
     if (!d.pt_active[p] || d.pt_coupled[p] >= 0) continue;
     double pd[kPointStride];
     load_record<kPointStride, true>(d.pdata + (size_t)p * kPointStride, pd);  // 320-byte records, 32-byte aligned
-    double h[3] = {0, 0, 0};
+    double tc[3] = {0, 0, 0};  // T_p y_c
 #pragma unroll
     for (int c = 0; c < NC; ++c) {
       const int r = d.cam_red[c];
       const double yc = r >= 0 ? y[r] : 0.0;
-      h[0] += pd[12 + 3 * c] * yc;
-      h[1] += pd[13 + 3 * c] * yc;
-      h[2] += pd[14 + 3 * c] * yc;
+      tc[0] += pd[12 + 3 * c] * yc;
+      tc[1] += pd[13 + 3 * c] * yc;
+      tc[2] += pd[14 + 3 * c] * yc;
     }
-    if (d.refine_poses) {  // sum_t V_t^T y_f, V_t recomputed from the track's A block, its frame entry and X
+    double h[3] = {0, 0, 0};
+    if (d.refine_poses) {  // sum_t V_t^T y_f, from the track's A block, its frame entry and X
       const double* __restrict__ frames = d.frames[cur];
       const double* X = d.points[cur] + 3 * (size_t)p;
       const double Xp[3] = {X[0], X[1], X[2]};
       for (int t = d.pt_trk_begin[p]; t < d.pt_trk_begin[p + 1]; ++t) {
         const int f = d.trk_frame[t];
-        double V[18], m[9], A[6];
+        const double* fe = frames + (size_t)f * kFrameStride;
+        double m[9], A[6];
         load_record<6, false>(d.rec[cur] + (size_t)t * rec_stride(NC), A);
-        track_v(A, frames + (size_t)f * kFrameStride, Xp, m, V);
-        const double* yf = y + 6 * f;
-#pragma unroll
-        for (int a = 0; a < 6; ++a) {
-          h[0] += V[3 * a] * yf[a];
-          h[1] += V[3 * a + 1] * yf[a];
-          h[2] += V[3 * a + 2] * yf[a];
-        }
+        track_m(fe, Xp, m);
+        track_vt_y_acc(A, fe, m, y + 6 * f, h);
       }
     }
     const double gp[3] = {pd[6], pd[7], pd[8]};
     const double rhs[3] = {gp[0] - h[0], gp[1] - h[1], gp[2] - h[2]};
     double yp[3];
     sym3_vec(pd, rhs, yp);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) yp[j] -= tc[j];
     const double* X = d.points[cur] + 3 * (size_t)p;
     double* Xc = d.points[cand] + 3 * (size_t)p;
 #pragma unroll

@@ -620,39 +620,120 @@ LFBA_HD double dot3_fma(double a0, double b0, double a1, double b1, double a2, d
   return fma(a2, b2, fma(a0, b0, a1 * b1));
 }
 
-// Pose-point coupling of one track, V = M^T A R (6 x 3, row-major: the pose x point block of J^T W J), recomputed
-// where it is used instead of being stored per track. A is the track's 3 x 3 block (upper: 00 01 02 11 12 22), fe its
-// frame-table entry (R, dR/da0..2), X the point. Also gives m, the 3 x 3 part of M = [dR0 X, dR1 X, dR2 X, I3]
-// (m[3 a + i] = (dR_a X)_i). Rows 3..5 are A R itself.
-LFBA_HD void track_v(const double A[6], const double* fe, const double* X, double m[9], double V[18]) {
+// ---- Pose-point coupling of one track, in the camera frame ----
+// The pose x point block of J^T W J of track t = (p, f) is V = M^T B, with B = A R (A the track's 3 x 3 block, R the
+// frame's rotation) and M = [dR0 X, dR1 X, dR2 X, I3] (3 x 6, d P_c / d pose). Every Schur term of a track has the form
+// M^T (3 x 3) M or (3 x NC)^T M, so the point is eliminated inside the 3 x 3 camera-frame block and the result is
+// projected onto the pose once; V and W = V Hpp^-1 are never formed. With Hi = (Hpp + D)^-1, K = B Hi and
+// T_p = Hi Hcp^T (3 x NC, stored per point by k_points):
+//     S_ff   += M^T (A - K B^T) M          g_f  += M^T (b - K g_p)          S_cf += (C - B T_p)^T M
+//     S_f1f2 -= M1^T (K1 B2^T) M2           y_p   = Hi (g_p - sum_t B^T M y_f) - T_p y_c
+// Every kernel builds these quantities with the helpers below, so all of them compute the same bits.
+// Storage: 3 x 3 symmetric as upper [00 01 02 11 12 22], general 3 x 3 row-major, m[3 a + i] = (dR_a X)_i.
+
+// m, the 3 x 3 part of M, from the frame-table entry fe (R, dR/da0..2) and the point X
+LFBA_HD void track_m(const double* fe, const double* X, double m[9]) {
 #pragma unroll
   for (int a = 0; a < 3; ++a) {
     const double* dR = fe + 9 * (a + 1);
 #pragma unroll
     for (int i = 0; i < 3; ++i) m[3 * a + i] = dot3_fma(dR[3 * i], X[0], dR[3 * i + 1], X[1], dR[3 * i + 2], X[2]);
   }
-  const double* R = fe;
+}
+// B = A R (A symmetric)
+LFBA_HD void track_b(const double A[6], const double* R, double B[9]) {
 #pragma unroll
   for (int j = 0; j < 3; ++j) {
-    V[9 + j] = dot3_fma(A[0], R[j], A[1], R[3 + j], A[2], R[6 + j]);
-    V[12 + j] = dot3_fma(A[1], R[j], A[3], R[3 + j], A[4], R[6 + j]);
-    V[15 + j] = dot3_fma(A[2], R[j], A[4], R[3 + j], A[5], R[6 + j]);
+    B[j] = dot3_fma(A[0], R[j], A[1], R[3 + j], A[2], R[6 + j]);
+    B[3 + j] = dot3_fma(A[1], R[j], A[3], R[3 + j], A[4], R[6 + j]);
+    B[6 + j] = dot3_fma(A[2], R[j], A[4], R[3 + j], A[5], R[6 + j]);
   }
+}
+// K = B Hi (Hi symmetric)
+LFBA_HD void mat3_sym3(const double B[9], const double Hi[6], double K[9]) {
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    const double* b = B + 3 * i;
+    K[3 * i] = dot3_fma(b[0], Hi[0], b[1], Hi[1], b[2], Hi[2]);
+    K[3 * i + 1] = dot3_fma(b[0], Hi[1], b[1], Hi[3], b[2], Hi[4]);
+    K[3 * i + 2] = dot3_fma(b[0], Hi[2], b[1], Hi[4], b[2], Hi[5]);
+  }
+}
+// G = K B2^T (general 3 x 3)
+LFBA_HD void mat3_mat3t(const double K[9], const double B2[9], double G[9]) {
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int j = 0; j < 3; ++j)
+      G[3 * i + j] = dot3_fma(K[3 * i], B2[3 * j], K[3 * i + 1], B2[3 * j + 1], K[3 * i + 2], B2[3 * j + 2]);
+}
+// A~ = A - K B^T, the track's camera-frame block with its point eliminated (symmetric: K B^T = B Hi B^T)
+LFBA_HD void track_atilde(const double A[6], const double B[9], const double K[9], double At[6]) {
+  int h = 0;
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int j = i; j < 3; ++j, ++h)
+      At[h] = A[h] - dot3_fma(K[3 * i], B[3 * j], K[3 * i + 1], B[3 * j + 1], K[3 * i + 2], B[3 * j + 2]);
+}
+// acc += M^T S M for a symmetric 3 x 3 S: the lower triangle of the 6 x 6 pose block, row-major ((a, c <= a) at
+// a (a + 1) / 2 + c)
+LFBA_HD void mt_sym_m_acc(const double m[9], const double S[6], double acc[21]) {
+  double Sm[9];
+#pragma unroll
+  for (int c = 0; c < 3; ++c) sym3_vec(S, m + 3 * c, Sm + 3 * c);
+  int h = 0;
+#pragma unroll
+  for (int a = 0; a < 6; ++a)
+#pragma unroll
+    for (int c = 0; c <= a; ++c, ++h) {
+      if (a < 3) acc[h] += dot3_fma(m[3 * a], Sm[3 * c], m[3 * a + 1], Sm[3 * c + 1], m[3 * a + 2], Sm[3 * c + 2]);
+      else if (c < 3) acc[h] += Sm[3 * c + a - 3];
+      else acc[h] += S[3 * (c - 3) - (c - 3) * (c - 2) / 2 + (a - 3)];  // upper (c - 3, a - 3)
+    }
+}
+// acc += s M^T v (6), s = +-1
+LFBA_HD void mt_vec_acc(const double m[9], const double v[3], double s, double acc[6]) {
+#pragma unroll
+  for (int a = 0; a < 3; ++a) acc[a] += s * dot3_fma(m[3 * a], v[0], m[3 * a + 1], v[1], m[3 * a + 2], v[2]);
+#pragma unroll
+  for (int i = 0; i < 3; ++i) acc[3 + i] += s * v[i];
+}
+// acc += M1^T G M2 (6 x 6 row-major) for a general 3 x 3 G
+LFBA_HD void mt_mat_m_acc(const double m1[9], const double G[9], const double m2[9], double acc[36]) {
+  double GM[18];  // G M2, 3 x 6 row-major
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+#pragma unroll
+    for (int b = 0; b < 3; ++b)
+      GM[6 * i + b] = dot3_fma(G[3 * i], m2[3 * b], G[3 * i + 1], m2[3 * b + 1], G[3 * i + 2], m2[3 * b + 2]);
+#pragma unroll
+    for (int b = 0; b < 3; ++b) GM[6 * i + 3 + b] = G[3 * i + b];
+  }
+#pragma unroll
+  for (int a = 0; a < 6; ++a)
+#pragma unroll
+    for (int b = 0; b < 6; ++b)
+      acc[6 * a + b] += a < 3 ? dot3_fma(m1[3 * a], GM[b], m1[3 * a + 1], GM[6 + b], m1[3 * a + 2], GM[12 + b])
+                              : GM[6 * (a - 3) + b];
+}
+// W = M^T K (6 x 3 row-major): V Hi for K = B Hi
+LFBA_HD void mt_mat(const double m[9], const double K[9], double W[18]) {
 #pragma unroll
   for (int a = 0; a < 3; ++a)
 #pragma unroll
-    for (int j = 0; j < 3; ++j)
-      V[3 * a + j] = dot3_fma(m[3 * a], V[9 + j], m[3 * a + 1], V[12 + j], m[3 * a + 2], V[15 + j]);
-}
-// W = V Hpp^-1 (6 x 3) from V and the inverse of the point's damped 3 x 3 block (upper triangle)
-LFBA_HD void track_w(const double Hi[6], const double V[18], double W[18]) {
+    for (int j = 0; j < 3; ++j) W[3 * a + j] = dot3_fma(m[3 * a], K[j], m[3 * a + 1], K[3 + j], m[3 * a + 2], K[6 + j]);
 #pragma unroll
-  for (int a = 0; a < 6; ++a) {
-    const double* v = V + 3 * a;
-    W[3 * a] = dot3_fma(Hi[0], v[0], Hi[1], v[1], Hi[2], v[2]);
-    W[3 * a + 1] = dot3_fma(Hi[1], v[0], Hi[3], v[1], Hi[4], v[2]);
-    W[3 * a + 2] = dot3_fma(Hi[2], v[0], Hi[4], v[1], Hi[5], v[2]);
-  }
+  for (int k = 0; k < 9; ++k) W[9 + k] = K[k];
+}
+// h += V^T y_f = R^T (A (M y_f)) for the pose step y_f (6) of the track's frame
+LFBA_HD void track_vt_y_acc(const double A[6], const double* R, const double m[9], const double* yf, double h[3]) {
+  double u[3], w[3];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) u[i] = yf[3 + i] + dot3_fma(m[i], yf[0], m[3 + i], yf[1], m[6 + i], yf[2]);
+  sym3_vec(A, u, w);
+#pragma unroll
+  for (int j = 0; j < 3; ++j) h[j] += dot3_fma(R[j], w[0], R[3 + j], w[1], R[6 + j], w[2]);
 }
 
 // distance constraint (src/BundleAdjustment/BundleAdjustment.h:262-267): r = (|p1 - p2| - d) / (sigma + 1e-6),
